@@ -1,6 +1,6 @@
 """bench.py -- BC train frames/s on N B200s (BASELINE.json metric), with roofline and CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...          (N > 1)
 
 One "step" = one optimisation step of the BC policy on `batch` frames per GPU:
@@ -211,6 +211,26 @@ WORKLOAD = ("ConvNet1 BC train step (BASELINE configs[1]), obs 4x256x256, 9 acti
             "u8 RGB frames staged on the device, sliding 4-frame window")
 
 
+def dump_outputs(out_dir, eng, bufs):
+    """What the last timed step handed its caller, as float32 .npy files: the loss, the logits of its batch, and the
+    parameters after its Adam update and the gradients of the step, both flattened in the module's parameter order.
+    With the peer exchange the gradients are this rank's, from the half of the double-buffered arena the last step wrote."""
+    import numpy as np
+    import torch
+    peer = eng.peer
+    if peer is not None:
+        half = peer.host_epoch & 1           # peer.current() is the half the NEXT step writes
+        grads = peer.buf[half * peer.n:(half + 1) * peer.n]
+    else:
+        grads = eng.grads
+    arrays = {"loss": bufs.loss.reshape(1), "logits": bufs.logits,
+              "params": torch.cat([eng.arena[o:o + n] for o, n in zip(eng.offsets, eng.sizes)]),
+              "grads": torch.cat([grads[o:o + n] for o, n in zip(eng.offsets, eng.sizes)])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def _event_ms(fn, reps=10, warm=3):
     import torch
     for _ in range(warm):
@@ -289,6 +309,9 @@ def run_b200(args):
     barrier()
     t_host1 = time.time()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        # taken here, before the passes below rewrite the loss, logits and gradient buffers
+        dump_outputs(args.dump_outputs, eng, ts.bufs)
     clocks = None
     if rank == 0:
         time.sleep(0.25)       # let the 100 ms sampler emit the rows that cover the end of the region
@@ -757,7 +780,11 @@ def main():
     ap.add_argument("--no-module", action="store_true", help="skip the device-resident module-path measurement")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="train workload: write what the last timed step computed (loss, logits, parameters, gradients) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "train"):
+        ap.error("--dump-outputs is implemented for --impl b200 --workload train")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "infer":

@@ -63,11 +63,13 @@ def golden_step(B, data_seed, path):
         opt.zero_grad(); l2.backward(); opt.step()
     after3 = flat(dict(net.named_parameters()))
     val = model.validation_step((x, y), 0)
+    # the parameters after the Adam steps go to a second file so that each stays under 1 MB
     np.savez_compressed(
         path, B=B, data_seed=data_seed, init=init, loss=float(loss.detach()), logits=logits, grads=grads,
-        after1=after1, after3=after3, val_loss_after3=float(val),
+        val_loss_after3=float(val),
         example_checksum=float(np.abs(example).sum()), example_logits=example_logits,
         logged_val=float(model.logged["val_loss"]))
+    np.savez_compressed(path.replace(".npz", "_adam.npz"), after1=after1, after3=after3)
     print(path, "loss", float(loss), "val", float(val))
 
 
@@ -138,11 +140,12 @@ def golden_resume_state(B, at_step, data_seed, path):
         opt.zero_grad(); loss.backward(); opt.step()
     named = dict(net.named_parameters())
     st = opt.state
+    # the Adam moments go to a second file so that each stays under 1 MB
+    np.savez_compressed(path, B=B, at_step=at_step, data_seed=data_seed, params=flat(named), last_loss=float(loss.detach()))
     np.savez_compressed(
-        path, B=B, at_step=at_step, data_seed=data_seed, params=flat(named),
+        path.replace(".npz", "_adam.npz"),
         exp_avg=np.concatenate([st[named[k]]["exp_avg"].reshape(-1).numpy() for k in O.PARAM_ORDER]),
-        exp_avg_sq=np.concatenate([st[named[k]]["exp_avg_sq"].reshape(-1).numpy() for k in O.PARAM_ORDER]),
-        last_loss=float(loss.detach()))
+        exp_avg_sq=np.concatenate([st[named[k]]["exp_avg_sq"].reshape(-1).numpy() for k in O.PARAM_ORDER]))
     print(path, "loss at resume", float(loss.detach()))
 
 

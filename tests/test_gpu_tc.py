@@ -218,7 +218,7 @@ def test_wgrad_tcgen05_matches_exact_f32_wgrad(B):
     eng.check_device_errors()
 
 
-def test_bf16_module_path_trains_like_the_reference(golden_dir):
+def test_bf16_module_path_trains_like_the_reference(golden_dir, tmp_path):
     """precision='bf16' through the Lightning-contract shells against the reference's 1k-step curve:
     per step on the plateau, then 800 steps from the reference's own state at step 200 (tests/curve_check.py)."""
     import os
@@ -230,6 +230,7 @@ def test_bf16_module_path_trains_like_the_reference(golden_dir):
     dev = torch.device("cuda", 0)
     g = np.load(os.path.join(golden_dir, "ref_curve_b8_1k.npz"))
     st = np.load(os.path.join(golden_dir, "ref_state_b8_step200.npz"))
+    st_adam = np.load(os.path.join(golden_dir, "ref_state_b8_step200_adam.npz"))
     B, steps, at = int(g["B"]), int(g["steps"]), int(st["at_step"])
     frames, labels = O.synth_frames(int(g["data_seed"]), steps * B + 4)
     lab = torch.from_numpy(labels).to(dev)
@@ -268,8 +269,8 @@ def test_bf16_module_path_trains_like_the_reference(golden_dir):
     for i, (n, p) in enumerate(net.named_parameters()):
         k = p.numel()
         sd[n] = torch.from_numpy(st["params"][off:off + k].copy()).view(p.shape)
-        adam[i] = dict(step=torch.tensor(float(at)), exp_avg=torch.from_numpy(st["exp_avg"][off:off + k].copy()).view(p.shape),
-                       exp_avg_sq=torch.from_numpy(st["exp_avg_sq"][off:off + k].copy()).view(p.shape))
+        adam[i] = dict(step=torch.tensor(float(at)), exp_avg=torch.from_numpy(st_adam["exp_avg"][off:off + k].copy()).view(p.shape),
+                       exp_avg_sq=torch.from_numpy(st_adam["exp_avg_sq"][off:off + k].copy()).view(p.shape))
         off += k
     net.load_state_dict(sd)
     opt = model.configure_optimizers()[0][0]
@@ -277,7 +278,7 @@ def test_bf16_module_path_trains_like_the_reference(golden_dir):
                                                             amsgrad=False, params=list(range(len(names))))]))
     got, _ = run(model, opt, at, steps)
     net.engine().check_device_errors()
-    np.save(os.path.join(os.environ.get("BC_TEST_OUT", "/tmp"), "curve_b8_1k_device_bf16.npy"), got)
+    np.save(os.path.join(os.environ.get("BC_TEST_OUT", str(tmp_path)), "curve_b8_1k_device_bf16.npy"), got)
     assert np.abs(got[:20] - ref[at:at + 20]).max() <= 5e-2 * ref[at:at + 20].max()       # still the same trajectory right after the resume
     check_curve(got, golden_dir, tol=2e-2, start=at)
 

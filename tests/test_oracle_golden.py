@@ -80,17 +80,18 @@ def test_explicit_backward_is_the_same_function(golden_dir, name):
 @pytest.mark.parametrize("name", ["ref_step_b4.npz", "ref_step_b1.npz"])
 def test_adam_three_steps(golden_dir, name):
     g = np.load(os.path.join(golden_dir, name))
+    adam = np.load(os.path.join(golden_dir, name.replace(".npz", "_adam.npz")))
     x, y = _batch(g)
     tr = O.OracleTrainer(_unflat(g["init"]))
     tr.step(x, y)
     a1 = _flat(tr.p)
     # Adam's first step moves every weight by ~lr*sign(g): compare the UPDATE, not just the value
-    d_ref = g["after1"].astype(np.float64) - g["init"].astype(np.float64)
+    d_ref = adam["after1"].astype(np.float64) - g["init"].astype(np.float64)
     d_got = a1 - g["init"].astype(np.float64)
     assert np.abs(d_got - d_ref).max() <= 2e-6  # |update| = 1e-3; f32 ulp of the params ~6e-8
     tr.step(x, y)
     tr.step(x, y)
-    assert np.abs(_flat(tr.p) - g["after3"].astype(np.float64)).max() <= 2e-5
+    assert np.abs(_flat(tr.p) - adam["after3"].astype(np.float64)).max() <= 2e-5
     val = float(O.cross_entropy(O.forward(tr.p, x), y))
     assert abs(val - float(g["val_loss_after3"])) <= 1e-4 * abs(float(g["val_loss_after3"]))
     assert float(g["logged_val"]) == float(g["val_loss_after3"])
