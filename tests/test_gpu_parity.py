@@ -185,7 +185,7 @@ def test_forward_and_loss_vs_reference_golden(golden_dir, name):
     assert _relerr(ex_logits, g["example_logits"]) <= REL_F32
 
 
-@pytest.mark.parametrize("B,seed", [(4, 0), (1, 1), (5, 2), (33, 3)])
+@pytest.mark.parametrize("B,seed", [(4, 0), (1, 1), (5, 2), (33, 3), (129, 4), (297, 5)])
 def test_gradients_given_device_routing(B, seed, golden_dir):
     dev = _dev()
     net = _net().to(dev)
