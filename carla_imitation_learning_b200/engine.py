@@ -126,11 +126,13 @@ def stage_frames(frames_u8: torch.Tensor, out: Optional[StagedBatch] = None, fra
     return out
 
 
-def stage_augmented(frames_u8: torch.Tensor, table: torch.Tensor, layout: str = "plain", frame_skip: int = 4):
+def stage_augmented(frames_u8: torch.Tensor, table: torch.Tensor, layout: str = "plain", frame_skip: int = 4, out=None):
     """EXTENSION (no counterpart in the reference): crop + colour jitter + normalise fused into the staging pass.
     frames (n, Hs, Ws, 3) u8 on the device with Hs, Ws >= 256; table (n, 8) f32 = data.augment_table(seed, ...) rows
     {crop_y, crop_x, brightness, contrast, saturation, mean, 1/std, -}. layout 'plain' -> (n,256,256) f32 gray planes
-    (use sliding_window() on them), 'tp' -> StagedBatch of Toeplitz-ready bf16 planes for precision='bf16'."""
+    (use sliding_window() on them), 'tp' -> StagedBatch of Toeplitz-ready bf16 planes for precision='bf16'.
+    `out` = persistent destination (a (n,256,256) f32 tensor for 'plain', a StagedBatch for 'tp'): a fixed-shape training
+    loop or a CUDA graph stages into the same buffers every step."""
     _require_cuda(frames_u8, "frames")
     if frames_u8.dtype != torch.uint8 or frames_u8.dim() != 4 or frames_u8.shape[-1] != 3 or not frames_u8.is_contiguous():
         raise ValueError("frames must be a contiguous (n,Hs,Ws,3) uint8 tensor")
@@ -141,11 +143,21 @@ def stage_augmented(frames_u8: torch.Tensor, table: torch.Tensor, layout: str = 
     if tuple(table.shape) != (n, 8):
         raise ValueError("the augmentation table is (n_frames, 8) float32")
     if layout == "plain":
-        out = torch.empty((n, H, W), dtype=torch.float32, device=frames_u8.device)
+        if out is None:
+            out = torch.empty((n, H, W), dtype=torch.float32, device=frames_u8.device)
+        elif (not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or tuple(out.shape) != (n, H, W)
+              or not out.is_contiguous() or out.device != frames_u8.device):
+            raise ValueError(f"out for layout 'plain' is a contiguous ({n},{H},{W}) float32 tensor on the frames' device")
         code, res = _lib.BC_F32, out
     elif layout == "tp":
-        out = torch.empty((n, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=frames_u8.device)
-        code, res = _lib.BC_BF16_TP, StagedBatch(out, None, frame_skip)
+        if out is None:
+            res = StagedBatch(torch.empty((n, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=frames_u8.device), None, frame_skip)
+        elif (not isinstance(out, StagedBatch) or tuple(out.tp.shape) != (n, _lib.TP_PLANE_ELEMS)
+              or out.tp.dtype != torch.bfloat16 or out.tp.device != frames_u8.device):
+            raise ValueError(f"out for layout 'tp' is a StagedBatch of {n} frames on the frames' device")
+        else:
+            res = out
+        code, out = _lib.BC_BF16_TP, res.tp
     else:
         raise ValueError("layout is 'plain' or 'tp'")
     if n:
@@ -435,7 +447,8 @@ class BCEngine:
         return self.w_packed.data_ptr() if self.conv_mode else None
 
     _ERRORS = {1: "a tcgen05 pipeline wait timed out inside a kernel (mbarrier protocol error)",
-               3: "a label outside [0, n_actions) reached the CrossEntropy kernel (nn.CrossEntropyLoss raises on it too)"}
+               3: "a label outside [0, n_actions) reached the CrossEntropy kernel (nn.CrossEntropyLoss raises on it too)",
+               4: "a command outside [0, n_branches) reached the branched heads (its output and gradient rows are zero)"}
 
     def check_device_errors(self) -> None:
         """Host-side check of the device error flag (synchronises; call outside the hot loop, e.g. at epoch end)."""
@@ -503,6 +516,27 @@ class BCEngine:
                 _lib.check(self.lib.bc_backward_overlap(C.byref(c), 1, s, side.cuda_stream, arr, flags), "bc_backward_overlap")
             else:
                 _lib.check(self.lib.bc_backward(C.byref(c), 1, s), "bc_backward")
+
+    def enqueue_trunk_forward(self, b: StepBuffers) -> None:
+        """conv1..4 (+ReLU+pool) of b's input into b.act on the current stream; no head (the branched heads follow)."""
+        c = self.ctx(b)
+        s = _stream_ptr()
+        with on_device(self.device):
+            for layer in range(4):
+                _lib.check(self.lib.bc_conv_relu_pool_fwd(C.byref(c), layer, s), f"conv{layer + 1} forward")
+
+    def enqueue_trunk_backward(self, b: StepBuffers) -> None:
+        """The conv trunk's backward from b.ghead (d loss / d act4, written by a head of the caller's: the branched heads)
+        on the current stream: weight and input gradients of conv4..conv2, conv1's weight gradient, and the reduction of
+        their partials into the engine's gradient arena. The arena's fc head segment is left untouched."""
+        c = self.ctx(b)
+        s = _stream_ptr()
+        with on_device(self.device):
+            for layer in (3, 2, 1):
+                _lib.check(self.lib.bc_conv_bwd_wgrad(C.byref(c), layer, s), "wgrad")
+                _lib.check(self.lib.bc_conv_bwd_dgrad(C.byref(c), layer, s), "dgrad")
+            _lib.check(self.lib.bc_conv_bwd_wgrad(C.byref(c), 0, s), "conv1 wgrad")
+            _lib.check(self.lib.bc_reduce_partials_range(C.byref(c), 1, 5, 0, s), "reduce [conv4..conv1]")
 
     tail_batch = 8       # serving: up to this batch conv3..head + argmax run as ONE cluster launch (bc_policy_tail). Measured crossover
                          # (bench.py --workload infer, profiles/r2G): 20.6-22.3 us against 26.3-26.6 us up to B = 8, 30.6 against 28.6 at B = 16

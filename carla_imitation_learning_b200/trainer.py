@@ -1,11 +1,13 @@
 """The training loop around the hot path: what `pl.Trainer(gpus=..., max_epochs=...).fit(model)` does for the
 behaviour-cloning block of the reference (/root/reference/train.py:106-129), for boxes without Lightning.
 
-Two layers:
+Three layers:
 
 * TrainStep -- one optimisation step for a static batch shape, straight on the engine (no autograd): stage -> conv1..4 ->
   head + CE -> backward -> [peer exchange] -> Adam as ONE CUDA graph per input slot. This is what bench.py times as `value`
   and what Trainer.fit uses when the module is a ConvNet1-backed Imitation with `cuda_graph: true`.
+* BranchedTrainStep -- the same for the command-conditioned ConvNet1Branched (one GPU): stage [+ augment] -> conv1..4 ->
+  branched heads + CE / L1 / MSE -> trunk backward -> Adam on the trunk and the branch arena, one CUDA graph per input slot.
 * Trainer -- epochs over model.train_dataloader() / val_dataloader() with the LightningModule hook order
   (training_step -> zero_grad -> backward -> optimizer.step; validation_step; *_epoch_end; scheduler.step once per epoch
   from training_epoch_end, imitation.py:57-60), ModelCheckpoint(monitor='val_loss', mode='min') in Lightning's .ckpt layout
@@ -21,7 +23,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .engine import BCEngine, StagedBatch, StepBuffers, stage_frames, stage_gray, sliding_window
+from .engine import BCEngine, StagedBatch, StepBuffers, stage_augmented, stage_frames, stage_gray, sliding_window
 from .optim import FusedAdam
 
 
@@ -124,6 +126,124 @@ class TrainStep:
         self.eng.check_device_errors()
         if self.dp is not None and hasattr(self.dp, "peer"):
             self.dp.peer.check()
+
+
+class BranchedTrainStep:
+    """stage [+ augment] -> conv1..4 -> branched heads + loss + backward -> trunk backward -> Adam on both arenas, for a
+    ConvNet1Branched and its MultiArenaAdam at a static batch, captured per input slot like TrainStep.
+
+    `step(frames_u8, table, command, target)`, all on the device: frames (B+4, Hs, Ws, 3) u8; table (B+4, 8) f32 rows of
+    data.augment_table when the step was built with src_hw = (Hs, Ws) (crop + colour jitter + normalise in the staging
+    kernel), None when src_hw is None (plain staging of 256x256 frames); command (B,) int64 branch ids; target (B,) int64
+    class ids for branch_loss 'ce', (B, n_out) f32 for 'l1' / 'mse'. The first call for a given buffer tuple runs
+    eagerly, the second captures a CUDA graph, later calls replay it. Returns the device loss cell, rewritten by the next
+    step. Nothing in step() synchronises the host; check() does."""
+
+    def __init__(self, net, optimizer, batch: int, *, src_hw=None, graph: bool = True, group=None):
+        if dist.is_initialized() and dist.get_world_size(group) > 1:
+            raise RuntimeError("BranchedTrainStep trains on one GPU: data-parallel training of the branched policy is not "
+                               "supported (the peer exchange drives a single parameter arena)")
+        children = getattr(optimizer, "children_", None)
+        if (children is None or len(children) != 2 or children[0]._arena_of is not net
+                or children[1]._arena_of is not net._bowner):
+            raise ValueError("BranchedTrainStep takes the net's MultiArenaAdam (net.configure_optimizer())")
+        self.net, self.opt, self.batch, self.graph = net, optimizer, int(batch), graph
+        self.trunk_opt, self.branch_opt = children
+        if self.batch < 1:
+            raise ValueError("batch must be at least 1")
+        self.src_hw = None if src_hw is None else (int(src_hw[0]), int(src_hw[1]))
+        if self.src_hw is not None and (self.src_hw[0] < 256 or self.src_hw[1] < 256):
+            raise ValueError(f"source frames {self.src_hw} are smaller than the 256x256 crop")
+        self.eng: BCEngine = net.engine()
+        eng, dev, B = self.eng, self.eng.device, self.batch
+        if eng.obs_size != 4:
+            raise ValueError("BranchedTrainStep stages 4-frame windows: obs_size must be 4")
+        if not net._barena.is_cuda or net._barena.device != dev:
+            raise RuntimeError("the branch arena must live on the trunk's device (net.to(device))")
+        self.bf16 = bool(eng.conv_mode)
+        if self.bf16:
+            self.staged = StagedBatch(torch.empty((B + 4, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev), None, 4)
+            self.bufs: StepBuffers = eng.alloc(B, self.staged, None, True)
+        else:
+            self.gray = torch.empty((B + 4, 256, 256), dtype=torch.float32, device=dev)
+            self.bufs = eng.alloc(B, sliding_window(self.gray), None, True)
+        n_part = int(_lib.lib().bc_head_branched_partials_floats(net.n_branches, net.n_actions))
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.hb = dict(out=torch.empty((B, net.n_actions), **f32), dout=torch.empty((B, net.n_actions), **f32),
+                       loss=torch.zeros((), **f32), grads=torch.zeros_like(net._barena),
+                       partials=torch.zeros(n_part, **f32))     # partial pads are never written: zeroed once
+        optimizer.prepare()
+        self._seen, self._graphs = set(), {}
+
+    # ------------------------------------------------------------------ pieces
+    def _check_inputs(self, frames_u8, table, command, target) -> None:
+        B, dev = self.batch, self.eng.device
+        hw = self.src_hw or (256, 256)
+        for t, what in ((frames_u8, "frames"), (command, "command"), (target, "target")):
+            if not isinstance(t, torch.Tensor) or t.device != dev:
+                raise ValueError(f"{what} must be a tensor on {dev}")
+        if frames_u8.dtype != torch.uint8 or tuple(frames_u8.shape) != (B + 4, *hw, 3) or not frames_u8.is_contiguous():
+            raise ValueError(f"frames must be a contiguous ({B + 4}, {hw[0]}, {hw[1]}, 3) uint8 tensor")
+        if self.src_hw is None:
+            if table is not None:
+                raise ValueError("this step was built without augmentation (src_hw=None): table must be None")
+        elif (not isinstance(table, torch.Tensor) or table.device != dev or table.dtype != torch.float32
+              or tuple(table.shape) != (B + 4, 8) or not table.is_contiguous()):
+            raise ValueError(f"table must be a contiguous ({B + 4}, 8) float32 tensor on {dev} (data.augment_table rows)")
+        if command.dtype != torch.int64 or tuple(command.shape) != (B,) or not command.is_contiguous():
+            raise ValueError(f"command must be a contiguous ({B},) int64 tensor of branch ids")
+        if self.net.branch_loss == "ce":
+            if target.dtype != torch.int64 or tuple(target.shape) != (B,) or not target.is_contiguous():
+                raise ValueError(f"CE targets are a contiguous ({B},) int64 tensor of class ids")
+        elif target.dtype != torch.float32 or tuple(target.shape) != (B, self.net.n_actions) or not target.is_contiguous():
+            raise ValueError(f"{self.net.branch_loss} targets are a contiguous ({B}, {self.net.n_actions}) float32 tensor")
+
+    def _stage(self, frames_u8, table) -> None:
+        if self.src_hw is not None:
+            stage_augmented(frames_u8, table, layout="tp" if self.bf16 else "plain", out=self.staged if self.bf16 else self.gray)
+        elif self.bf16:
+            stage_frames(frames_u8, out=self.staged)
+        else:
+            stage_gray(frames_u8, out=self.gray)
+
+    def _enqueue(self, frames_u8, table, command, target) -> None:
+        self._stage(frames_u8, table)
+        self.eng.enqueue_trunk_forward(self.bufs)
+        self.net._head(self.bufs, self.hb, command, target, 3)      # outputs, loss, dout, branch gradients, ghead
+        self.eng.enqueue_trunk_backward(self.bufs)
+        self.trunk_opt.step_flat(self.eng.grads)
+        self.branch_opt.step_flat(self.hb["grads"])
+
+    # ------------------------------------------------------------------ step
+    def step(self, frames_u8: torch.Tensor, table: Optional[torch.Tensor], command: torch.Tensor,
+             target: torch.Tensor) -> torch.Tensor:
+        """Enqueue one optimisation step; returns the (device) loss cell, rewritten by the next step."""
+        self._check_inputs(frames_u8, table, command, target)
+        self.eng.ensure_packed()
+        key = (frames_u8.data_ptr(), None if table is None else table.data_ptr(), command.data_ptr(), target.data_ptr())
+        g = self._graphs.get(key) if self.graph else None
+        if g is None and self.graph and key in self._seen:
+            self.opt.prepare()
+            g = self._graphs[key] = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._enqueue(frames_u8, table, command, target)
+        if g is not None:
+            self.opt.prepare()            # an LR milestone reaches the device scalars the captured Adam kernels read
+            g.replay()
+        else:
+            self._seen.add(key)
+            self.opt.prepare()
+            self._enqueue(frames_u8, table, command, target)
+        return self.hb["loss"]
+
+    @property
+    def out(self) -> torch.Tensor:
+        """(B, n_out) outputs of the commanded branches in the last step (before its update)."""
+        return self.hb["out"]
+
+    def check(self) -> None:
+        """Raise if a device-side bounded wait expired, a label (CE) or a command was out of range (synchronises)."""
+        self.eng.check_device_errors()
 
 
 def arena_checksum(arena: torch.Tensor) -> int:

@@ -152,8 +152,8 @@ int bc_loss_reduce(const bc_ctx* c, void* stream);                 /* head CTAs'
 
 /* ---- Launch ordering contract (programmatic dependent launch). Every kernel of this library is launched with programmatic
  * stream serialisation. Kernels that READ parameters -- the conv / dgrad kernels (their bf16 operand images in w_packed), the
- * head (fc weights) and the optimiser kernels (params, moments, state) -- fetch them BEFORE griddepcontrol.wait, under the
- * previous kernel's tail. That is sound because the kernels that WRITE parameters, moments, state or w_packed (bc_adam_step,
+ * head (fc weights), the branched heads (bc_head_branched: the commanded branch's weights in the branch arena) and the
+ * optimiser kernels (params, moments, state) -- fetch them BEFORE griddepcontrol.wait, under the previous kernel's tail. That is sound because the kernels that WRITE parameters, moments, state or w_packed (bc_adam_step,
  * bc_adam_tick_step, bc_adam_step_exchange, bc_pack_weights) release their dependents only after their last write. A caller
  * that writes these buffers itself must do so with ordinary (fully serialising) launches or copies -- torch ops are --
  * and never from a kernel of its own that calls griddepcontrol.launch_dependents before its last write. */
@@ -218,7 +218,9 @@ int bc_scale_inplace(float* v, int64_t n, const float* scale_dev, void* stream);
  * params / grads: G x head_len floats, per branch in the order of the arena's head segment [fc.4 w,b | fc.2 w,b | fc.0 w,b]
  * (bc_head_branched_layout gives the per-branch offsets in state_dict order 0.weight 0.bias 2.weight 2.bias 4.weight 4.bias).
  * feat = bc_ctx.act[3] of the conv trunk, gfeat = bc_ctx.ghead for the trunk's backward. mode bit0: loss + dout from
- * labels/targets; bit1: backward from dout (grads, gfeat); 0 = outputs only. */
+ * labels/targets; bit1: backward from dout (grads, gfeat); 0 = outputs only. A command outside [0, n_branches) sets
+ * *err_flag = 4 and leaves zeros in that sample's rows: out, dout (bit0) and gfeat (bit1), so the sample adds nothing to the
+ * trunk's backward and no stale gradient row reaches it. */
 typedef struct {
     int32_t n_branches, n_out, batch, loss_kind;
     const float* feat;        /* (B,128)                               */

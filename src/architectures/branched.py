@@ -164,10 +164,8 @@ class ConvNet1Branched(ConvNet1):
     def _trunk_forward(self, x, backward: bool):
         eng = self.engine()
         bufs = eng.alloc(x.shape[0], x, None, backward)
-        c = eng.ctx(bufs)
         with torch.cuda.device(eng.device):
-            for layer in range(4):
-                _lib.check(eng.lib.bc_conv_relu_pool_fwd(C.byref(c), layer, _stream_ptr()), f"conv{layer + 1} forward")
+            eng.enqueue_trunk_forward(bufs)
         return bufs
 
     @torch.no_grad()
@@ -199,14 +197,8 @@ class _BranchedLoss(torch.autograd.Function):
         eng = net.engine()
         hb["dout"].mul_(gloss)
         net._head(bufs, hb, ctx.command, None, 2)
-        c = eng.ctx(bufs)
-        s = _stream_ptr()
         with torch.cuda.device(eng.device):
-            for layer in (3, 2, 1):
-                _lib.check(eng.lib.bc_conv_bwd_wgrad(C.byref(c), layer, s), "wgrad")
-                _lib.check(eng.lib.bc_conv_bwd_dgrad(C.byref(c), layer, s), "dgrad")
-            _lib.check(eng.lib.bc_conv_bwd_wgrad(C.byref(c), 0, s), "conv1 wgrad")
-            _lib.check(eng.lib.bc_reduce_partials_range(C.byref(c), 1, 5, 0, s), "reduce [conv4..conv1]")
+            eng.enqueue_trunk_backward(bufs)
         flat = eng._last_flat = eng.grad_view().clone()
         bflat = hb["grads"].clone()
         tg = [flat[p._bc_offset:p._bc_offset + p.numel()].view(p.shape) for p in net.trunk_parameters()]
@@ -233,6 +225,14 @@ class MultiArenaAdam(torch.optim.Optimizer):
             c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
             c.step()
         return loss
+
+    def prepare(self) -> None:
+        """Push param_groups[0]['lr'] into every child's device scalar (allocating their state on the first call). Call
+        before capturing a CUDA graph that holds the Adam launches and before every replay, so a MultiStepLR milestone
+        reaches the captured kernels."""
+        for c in self.children_:
+            c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
+            c.prepare()
 
     def zero_grad(self, set_to_none: bool = True) -> None:
         for c in self.children_:
