@@ -126,22 +126,41 @@ def stage_frames(frames_u8: torch.Tensor, out: Optional[StagedBatch] = None, fra
     return out
 
 
+def _check_augment_table(table: torch.Tensor, hs: int, ws: int) -> None:
+    """Rows {crop_y, crop_x, brightness, contrast, saturation, mean, 1/std, -} of a host f32 table: a crop outside the
+    source would make the staging kernel read outside the frames."""
+    t = table[:, :7].double()
+    if not bool(torch.isfinite(t).all()):
+        raise ValueError("the augmentation table has a non-finite entry")
+    crop = t[:, :2]
+    if not torch.equal(crop, crop.floor()):
+        raise ValueError("the augmentation table's crop offsets must be integers")
+    if t.shape[0] and (float(crop.min()) < 0 or float(crop[:, 0].max()) > hs - H or float(crop[:, 1].max()) > ws - W):
+        raise ValueError(f"the augmentation table's crop offsets must lie in [0, {hs - H}] x [0, {ws - W}] for {hs}x{ws} sources")
+
+
 def stage_augmented(frames_u8: torch.Tensor, table: torch.Tensor, layout: str = "plain", frame_skip: int = 4, out=None):
     """EXTENSION (no counterpart in the reference): crop + colour jitter + normalise fused into the staging pass.
     frames (n, Hs, Ws, 3) u8 on the device with Hs, Ws >= 256; table (n, 8) f32 = data.augment_table(seed, ...) rows
     {crop_y, crop_x, brightness, contrast, saturation, mean, 1/std, -}. layout 'plain' -> (n,256,256) f32 gray planes
     (use sliding_window() on them), 'tp' -> StagedBatch of Toeplitz-ready bf16 planes for precision='bf16'.
     `out` = persistent destination (a (n,256,256) f32 tensor for 'plain', a StagedBatch for 'tp'): a fixed-shape training
-    loop or a CUDA graph stages into the same buffers every step."""
+    loop or a CUDA graph stages into the same buffers every step.
+    A host table is checked before it is copied: integral crop offsets in [0, Hs-256] x [0, Ws-256] and finite factors,
+    else ValueError and nothing is launched. A device table is not read back (that would synchronise every step): its
+    rows are the caller's contract, as for BranchedTrainStep."""
     _require_cuda(frames_u8, "frames")
     if frames_u8.dtype != torch.uint8 or frames_u8.dim() != 4 or frames_u8.shape[-1] != 3 or not frames_u8.is_contiguous():
         raise ValueError("frames must be a contiguous (n,Hs,Ws,3) uint8 tensor")
     n, hs, ws, _ = frames_u8.shape
     if hs < H or ws < W:
         raise ValueError(f"source frames {hs}x{ws} are smaller than the {H}x{W} crop")
-    table = table.to(device=frames_u8.device, dtype=torch.float32).contiguous()
     if tuple(table.shape) != (n, 8):
         raise ValueError("the augmentation table is (n_frames, 8) float32")
+    if table.device.type == "cpu":
+        table = table.to(dtype=torch.float32)
+        _check_augment_table(table, hs, ws)
+    table = table.to(device=frames_u8.device, dtype=torch.float32).contiguous()
     if layout == "plain":
         if out is None:
             out = torch.empty((n, H, W), dtype=torch.float32, device=frames_u8.device)

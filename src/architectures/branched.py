@@ -208,12 +208,25 @@ class _BranchedLoss(torch.autograd.Function):
 
 class MultiArenaAdam(torch.optim.Optimizer):
     """One torch.optim.Optimizer over several flat arenas: a FusedAdam (one fused launch) per arena; the learning rate of
-    param_groups[0] -- what MultiStepLR drives -- is handed to all of them."""
+    param_groups[0] -- what MultiStepLR drives -- is handed to all of them.
+
+    The moments and step counts live in the children. self.state exposes their per-parameter views, and state_dict() /
+    load_state_dict() use one parameter index space over all arenas: the layout torch.optim.Adam(list(net.parameters()))
+    writes, so a checkpoint of either optimiser restores into the other."""
 
     def __init__(self, param_lists, lr: float = 1e-3):
         params = [p for ps in param_lists for p in ps]
         super().__init__(params, dict(lr=lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False))
         self.children_ = [FusedAdam(list(ps), lr=lr) for ps in param_lists]
+        self._linked = [None] * len(self.children_)
+
+    def _link_state(self) -> None:
+        """self.state[p] = the child's torch.optim.Adam-compatible views (FusedAdam._bind), refreshed when a child rebinds."""
+        for i, c in enumerate(self.children_):
+            if c._bound is not None and self._linked[i] is not c._bound:
+                for p in c._params:
+                    self.state[p] = c.state[p]
+                self._linked[i] = c._bound
 
     @torch.no_grad()
     def step(self, closure=None):
@@ -224,6 +237,7 @@ class MultiArenaAdam(torch.optim.Optimizer):
         for c in self.children_:
             c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
             c.step()
+        self._link_state()
         return loss
 
     def prepare(self) -> None:
@@ -233,7 +247,30 @@ class MultiArenaAdam(torch.optim.Optimizer):
         for c in self.children_:
             c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
             c.prepare()
+        self._link_state()
 
     def zero_grad(self, set_to_none: bool = True) -> None:
         for c in self.children_:
             c.zero_grad(set_to_none)
+
+    # ------------------------------------------------------------------ checkpoints
+    def state_dict(self):
+        """torch.optim.Adam's layout: state[i] = {step, exp_avg, exp_avg_sq} of param_groups[0]['params'][i]."""
+        self._link_state()
+        return super().state_dict()
+
+    def load_state_dict(self, state_dict) -> None:
+        """Accepts what state_dict() writes and a torch.optim.Adam state_dict over the same parameter list (its groups'
+        indices, in order, are matched to param_groups[0]['params']). Each child gets its parameters' moments and the step
+        count (FusedAdam.load_state_dict); the restored learning rate reaches every child's device scalar."""
+        groups = state_dict["param_groups"]
+        ids = [pid for g in groups for pid in g["params"]]
+        own = self.param_groups[0]["params"]
+        if len(ids) != len(own):
+            raise ValueError(f"the optimiser state holds {len(ids)} parameters, this optimiser has {len(own)}")
+        gid = {id(p): pid for p, pid in zip(own, ids)}
+        for c in self.children_:
+            c.load_state_dict({"state": state_dict["state"],
+                               "param_groups": [{"params": [gid[id(p)] for p in c._params], "lr": groups[0]["lr"]}]})
+        self.param_groups[0]["lr"] = groups[0]["lr"]
+        self.prepare()
