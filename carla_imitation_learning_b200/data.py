@@ -79,7 +79,13 @@ class SequentialFrames:
     layout='tp' (the bf16 tensor-core mode), a StagedBatch of Toeplitz-ready planes written by the same
     single staging pass; y the (b,) int64 labels of the frames that follow each window. The last batch may be
     short (the reference's DataLoader has no drop_last). Host frames are pinned; chunk k+1's
-    H2D copy and staging run on a side stream while the trainer consumes chunk k.
+    H2D copy runs on a side stream while the trainer consumes chunk k.
+
+    x and y are views of two rotating device slots, not copies. A yielded batch stays valid until the consumer has asked
+    the same iterator for two more: work enqueued on the consumer's current stream before that second request reads
+    batch k (so two micro-batches may be accumulated across one next()); the request that hands out batch k + 2
+    restages the slot, and a new iterator starts again from the first slot. Keep a batch longer, or read it from another
+    stream, and clone it first.
     """
 
     def __init__(self, frames_u8: np.ndarray, labels: np.ndarray, batch_size: int = 64, frame_skip: int = 4,
@@ -119,16 +125,14 @@ class SequentialFrames:
         return (self.n_samples + self.batch_size - 1) // self.batch_size
 
     def _produce(self, k: int, slot: int) -> torch.cuda.Event:
-        """H2D of chunk k's frames and labels into raw slot `slot` on the copy stream (nothing else runs there: uploads go
-        back to back; the staging kernel runs on the consumer's stream right before the batch is handed out)."""
+        """H2D of chunk k's frames into raw slot `slot` on the copy stream (nothing else runs there: uploads go back to
+        back; the staging kernel runs on the consumer's stream right before the batch is handed out)."""
         lo = k * self.batch_size
         hi = min(lo + self.batch_size, self.n_samples) + self.frame_skip
         with torch.cuda.stream(self._copy_stream):
             if self._staged[slot] is not None:
                 self._copy_stream.wait_event(self._staged[slot])       # the staging pass that last read this raw slot
             self._raw[slot][:hi - lo].copy_(self.frames[lo:hi], non_blocking=True)
-            nb = hi - lo - self.frame_skip
-            self._lab[slot][:nb].copy_(self.labels[lo + self.frame_skip: lo + self.frame_skip + nb], non_blocking=True)
             ev = torch.cuda.Event()
             ev.record(self._copy_stream)
         return ev
@@ -140,6 +144,10 @@ class SequentialFrames:
             stage_frames(self._raw[slot][:hi - lo], out=StagedBatch(self._gray[slot][:hi - lo], None, self.frame_skip))
         else:
             stage_gray(self._raw[slot][:hi - lo], out=self._gray[slot][:hi - lo])
+        # the labels are copied on the consumer's stream too (device to device): a step of batch k - 2 still queued there
+        # reads this slot's previous labels, and the copy stream would not wait for it
+        nb = hi - lo - self.frame_skip
+        self._lab[slot][:nb].copy_(self.labels[lo + self.frame_skip: lo + self.frame_skip + nb])
         if self._staged[slot] is None:
             self._staged[slot] = torch.cuda.Event()
         self._staged[slot].record(cur)

@@ -433,7 +433,10 @@ class BCEngine:
             if torch.cuda.is_current_stream_capturing():
                 raise RuntimeError("create the engine's side stream before capturing (run one eager step first)")
             with on_device(self.device):
-                side = torch.cuda.Stream(self.device)
+                # torch hands out pool streams round robin, 32 per priority: a default-priority side stream becomes the
+                # CUDA-graph capture stream again once 32 more streams have been created (one per SequentialFrames
+                # loader), and bc_backward_overlap refuses side == main. The high-priority pool holds no such stream.
+                side = torch.cuda.Stream(self.device, priority=-1)
                 evs = [torch.cuda.Event() for _ in range(4)]
                 for e in evs:
                     e.record()                      # torch creates the cudaEvent lazily: force it now
