@@ -103,8 +103,10 @@ __global__ void __launch_bounds__(NT) head_kernel(const HeadArgs a) {
         if (tid < NA) a.logits[(size_t)b * NA + tid] = s_z[tid];
         if (a.actions && warp == 0) {
             const float z = lane < NA ? s_z[lane] : -INFINITY;
-            const float m = bc::warp_max(z);
-            const unsigned hit = __ballot_sync(0xffffffffu, lane < NA && z == m);   // first maximum, like torch.argmax
+            const float m = bc::warp_max(z);                                         // fmaxf: drops NaN
+            // like torch.argmax: the first NaN if there is one (NaN counts as the maximum), else the first maximum
+            const unsigned nan = __ballot_sync(0xffffffffu, lane < NA && isnan(z));
+            const unsigned hit = nan ? nan : __ballot_sync(0xffffffffu, lane < NA && z == m);
             if (lane == 0) a.actions[b] = hit ? (int64_t)(__ffs((int)hit) - 1) : 0;
         }
         if (!do_ce && !do_bwd) continue;
@@ -187,8 +189,9 @@ __global__ void argmax_kernel(const float* __restrict__ logits, int64_t* __restr
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     const float* z = logits + (size_t)b * NA;
+    // like torch.argmax: the first NaN if there is one (NaN counts as the maximum), else the first maximum
     float best = z[0]; int idx = 0;
-    for (int c = 1; c < NA; ++c) if (z[c] > best) { best = z[c]; idx = c; }  // first maximum, like torch.argmax
+    for (int c = 1; c < NA && !isnan(best); ++c) if (z[c] > best || isnan(z[c])) { best = z[c]; idx = c; }
     out[b] = idx;
 }
 

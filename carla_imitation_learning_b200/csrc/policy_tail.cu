@@ -18,7 +18,8 @@
 //            cluster barrier every CTA pulls the other seven CTAs' 128 pooled values through distributed shared memory;
 //   phase C  conv4 for the CTA's 16 channels: a thread owns (channel, 4 of the 64 input channels) for all 2x2 conv pixels,
 //            16-lane xor tree, + bias, ReLU, max -> the 16 features go to CTA 0's shared memory;
-//   phase D  CTA 0: the three Linear layers on all 256 threads (rows split over neighbouring lanes), logits, first maximum.
+//   phase D  CTA 0: the three Linear layers on all 256 threads (rows split over neighbouring lanes), logits, greedy action
+//            (torch.argmax's rule: the first NaN, else the first maximum).
 // Two cluster barriers per sample; no global-memory round trip between the layers.
 #include "bc_common.cuh"
 #include "trace.cuh"
@@ -338,8 +339,10 @@ __global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a) {
     if (tid < NA) a.logits[(size_t)b * NA + tid] = s_z[tid];
     if (warp == 0 && a.actions) {
         const float z = lane < NA ? s_z[lane] : -INFINITY;
-        const float m = bc::warp_max(z);
-        const unsigned hit = __ballot_sync(0xffffffffu, lane < NA && z == m);   // first maximum, like torch.argmax
+        const float m = bc::warp_max(z);                                         // fmaxf: drops NaN
+        // like torch.argmax: the first NaN if there is one (NaN counts as the maximum), else the first maximum
+        const unsigned nan = __ballot_sync(0xffffffffu, lane < NA && isnan(z));
+        const unsigned hit = nan ? nan : __ballot_sync(0xffffffffu, lane < NA && z == m);
         if (lane == 0) a.actions[b] = hit ? (int64_t)(__ffs((int)hit) - 1) : 0;
     }
     TRACE(9, 0);

@@ -191,12 +191,15 @@ typedef struct {
 int bc_adam_step_exchange(float* params, float* exp_avg, float* exp_avg_sq, double* state9, int64_t n, const bc_peer* peer,
                           int64_t lo, int64_t hi, int bucket, int publish, void* w_packed, int obs_size, int n_actions, void* stream);
 
-/* ---- K12: Imitation.forward + argmax (imitation.py:34-36, src/data/stat.py:41) */
+/* ---- K12: Imitation.forward + argmax (imitation.py:34-36, src/data/stat.py:41). Every greedy action of this library
+ * (bc_argmax, bc_forward_act on both paths) follows torch.argmax: the index of the first NaN of the row if it has one (NaN
+ * counts as the maximum), else the index of the first maximum (ties go to the lowest index; a row of -inf gives 0). */
 int bc_argmax(const float* logits, int64_t* actions, int batch, int n_actions, void* stream);
 
 /* ---- K13: the policy forward for closed-loop serving (BASELINE configs[4]; imitation.py:34-36 + the argmax of
  * src/data/stat.py:41), greedy actions (batch) int64 out, no separate argmax launch.
- * bc_forward_act, tail = 0: bc_forward with the first-maximum action taken inside the head kernel.
+ * bc_forward_act, tail = 0: bc_forward with the action taken inside the head kernel (torch.argmax's rule, K12 above: the
+ *   first NaN, else the first maximum; the same on both paths).
  * tail = 1 (batch <= BC_POLICY_TAIL_MAX_BATCH; faster up to batch 8 on B200, where the forward is a chain of launch latencies):
  *   conv1, conv2 as in bc_forward, then bc_policy_tail = conv3 + ReLU + pool, conv4 + ReLU + pool, the three Linear layers and the
  *   argmax in ONE launch (an 8-CTA thread-block cluster per sample, exact f32 FFMA on the f32 master weights in both modes,

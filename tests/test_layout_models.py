@@ -251,10 +251,22 @@ def test_dgrad_toeplitz_in_n_fold(hin, ks, wp):
 
 
 def test_policy_tail_thread_mapping_reproduces_conv3_conv4_head():
+    _policy_tail_thread_model(9)
+
+
+@pytest.mark.parametrize("NA", [1, 16])
+def test_policy_tail_thread_mapping_at_the_narrowest_and_widest_head(NA):
+    """The same model at n_actions 1 and 16: the fc.4 load covers exactly NA rows and the row clamp cc of lanes c >= NA."""
+    _policy_tail_thread_model(NA)
+
+
+def _policy_tail_thread_model(NA):
     """csrc/policy_tail.cu written out thread by thread in numpy: the shared-memory plan (padded channel pitches W3P / W4P / PTP /
     A3P), the (2 channels x pooled row x 2 input channels) register tile of conv3, the partial reduction split over (px, dy, h, g)
     lanes, the pull all-gather across the 8 CTAs of a cluster, conv4's (channel, 4 input channels) threads with the 16-lane fold, and
-    the lane-split Linear layers with their rotated inner index -- against the plain convolutions / matrix products (integers, exact)."""
+    the lane-split Linear layers with their rotated inner index -- against the plain convolutions / matrix products (integers, exact).
+    Every head width loads its own NA rows of fc.4 (tid < NA * 8) into a shared-memory region that holds BC_MAX_ACTIONS = 16 rows,
+    and the lanes of rows c >= NA read the clamped row NA - 1."""
     rng = np.random.default_rng(5)
     W3P, W4P, PTP, A3P = 516, 592, 36, 20
     act2 = rng.integers(-3, 4, size=(32, 12, 12)).astype(np.int64)
@@ -264,7 +276,6 @@ def test_policy_tail_thread_mapping_reproduces_conv3_conv4_head():
     b4 = rng.integers(-5, 6, size=128).astype(np.int64)
     f0 = rng.integers(-2, 3, size=(64, 128)).astype(np.int64); g0 = rng.integers(-3, 4, size=64).astype(np.int64)
     f2 = rng.integers(-2, 3, size=(32, 64)).astype(np.int64); g2 = rng.integers(-3, 4, size=32).astype(np.int64)
-    NA = 9
     f4 = rng.integers(-2, 3, size=(NA, 32)).astype(np.int64); g4 = rng.integers(-3, 4, size=NA).astype(np.int64)
 
     # ---- reference: conv (valid) + ReLU + floor-mode 2x2 max pool, twice; three Linear layers
@@ -378,18 +389,27 @@ def test_policy_tail_thread_mapping_reproduces_conv3_conv4_head():
         p = p + p[tid ^ offx]
     s_h2 = np.zeros(32, np.int64); s_h2[j[e8 == 0]] = np.maximum(p + g2[j], 0)[e8 == 0]
     assert np.array_equal(s_h2, h2)
+    # fc.4: float4 word tid of the weight for tid < NA * 8 (rows beyond NA stay whatever shared memory held), bias for tid < NA
+    MAXA = 16
+    s_w4 = np.full(MAXA * 32, 10 ** 9, np.int64)
+    has4 = tid < NA * 8
+    for e in range(4):
+        s_w4[4 * tid[has4] + e] = f4.reshape(-1)[4 * tid[has4] + e]
+    s_b4 = np.full(MAXA, 10 ** 9, np.int64)
+    s_b4[tid[tid < NA]] = g4[tid[tid < NA]]
     c, e8 = tid >> 3, tid & 7
     cc = np.minimum(c, NA - 1)
     p = np.zeros(256, np.int64)
     for i in range(4):
         k = (i + c) & 3
-        p += f4.reshape(-1)[cc * 32 + e8 * 4 + k] * s_h2[e8 * 4 + k]
+        p += s_w4[cc * 32 + e8 * 4 + k] * s_h2[e8 * 4 + k]
     for offx in (1, 2, 4):
         p = p + p[tid ^ offx]
     z = np.zeros(NA, np.int64)
     ok = (e8 == 0) & (c < NA)
-    z[c[ok]] = (p + g4[cc])[ok]
+    z[c[ok]] = (p + s_b4[cc])[ok]
     assert np.array_equal(z, ref_z)
-    # first maximum: ballot of the lanes that hold the maximum, lowest set bit
-    m = z.max()
-    assert int(np.flatnonzero(z == m)[0]) == int(np.argmax(z))
+    # greedy action on warp 0: ballot of the lanes < NA that hold the maximum, lowest set bit (no NaN among integers)
+    zl = np.where(lane < NA, np.concatenate([z, np.zeros(32, np.int64)])[lane], np.iinfo(np.int64).min)[:32]
+    hit = (lane[:32] < NA) & (zl == zl.max())
+    assert int(np.flatnonzero(hit)[0]) == int(np.argmax(ref_z))
