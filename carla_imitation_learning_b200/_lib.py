@@ -88,6 +88,8 @@ EXPORTS = {
     "bc_head_branched": (C.c_int, [C.POINTER(BcBranched), C.c_int, C.c_void_p]),
     "bc_head_branched_partials_floats": (C.c_size_t, [C.c_int, C.c_int]),
     "bc_head_branched_layout": (C.c_int64, [C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "bc_forward_branched_act": (C.c_int, [C.POINTER(BcCtx), C.POINTER(BcBranched), C.c_void_p, C.c_int, C.c_void_p]),
+    "bc_policy_tail_branched": (C.c_int, [C.POINTER(BcCtx), C.POINTER(BcBranched), C.c_void_p, C.c_void_p]),
     "bc_scale_inplace": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "bc_tc_gemm_selftest": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bc_tc_mma_bench": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -16,6 +16,8 @@
 // single head (head.cu): the branch arena is written only by torch ops and by bc_adam_tick_step, which releases its
 // dependents after its last write (include/bc_b200.h, launch ordering). A command outside [0, G) raises flag 4; that
 // sample's out row (and dout row with the loss, gfeat row with the backward) is written as zeros.
+// Serving (bc_forward_branched_act, tail = 0): with `actions` set (mode 0 only), warp 0 also takes each sample's greedy
+// action from its outputs, by the ballot code of the single-head tail (policy_tail.cu); an out-of-range command gets 0.
 #include "bc_common.cuh"
 
 namespace {
@@ -44,6 +46,7 @@ __host__ inline HeadLayout head_layout(int na) {      // the order of the arena'
 struct BrArgs {
     const float* feat; const int64_t* cmd; const int64_t* y; const float* tgt; const float* params;
     float* out; float* dout; float* gfeat; float* part; float* loss_part;
+    int64_t* actions;                         // (B,) greedy actions over out, or NULL (mode 0 only)
     HeadLayout L;
     int B, NA, G, nb, mode, kind;
     float loss_scale;
@@ -112,6 +115,7 @@ __global__ void __launch_bounds__(NT) head_branched_kernel(const BrArgs a) {
             if (b < a.B && (cmd[k] < 0 || cmd[k] >= a.G) && reporter) {   // reported; the sample leaves zero rows behind
                 if (a.err) atomicExch(a.err, 4);
                 for (int j = 0; j < NA; ++j) a.out[(size_t)b * NA + j] = 0.f;
+                if (a.actions) a.actions[b] = 0;
                 if (do_loss) for (int j = 0; j < NA; ++j) a.dout[(size_t)b * NA + j] = 0.f;
                 if (do_bwd) for (int j = 0; j < 128; ++j) a.gfeat[(size_t)b * 128 + j] = 0.f;
             }
@@ -168,6 +172,14 @@ __global__ void __launch_bounds__(NT) head_branched_kernel(const BrArgs a) {
             }
             __syncthreads();
             if (tid < NA) a.out[(size_t)b * NA + tid] = s_z[tid];
+            if (warp == 0 && a.actions) {
+                const float z = lane < NA ? s_z[lane] : -INFINITY;
+                const float m = bc::warp_max(z);                                 // fmaxf: drops NaN
+                // like torch.argmax: the first NaN if there is one (NaN counts as the maximum), else the first maximum
+                const unsigned nan = __ballot_sync(0xffffffffu, lane < NA && isnan(z));
+                const unsigned hit = nan ? nan : __ballot_sync(0xffffffffu, lane < NA && z == m);
+                if (lane == 0) a.actions[b] = hit ? (int64_t)(__ffs((int)hit) - 1) : 0;
+            }
             if (!do_loss && !do_bwd) continue;
             if (warp == 0) {
                 if (do_loss) {
@@ -292,8 +304,10 @@ extern "C" size_t bc_head_branched_partials_floats(int n_branches, int n_out) {
     return (size_t)n_branches * nb * l.len + 32 * (((size_t)n_branches * nb + 31) / 32);
 }
 
-extern "C" int bc_head_branched(const bc_branched* h, int mode, void* stream) {
-    BC_CHECK_ARG(h && h->feat && h->command && h->params && h->out && h->partials, "bc_head_branched: null buffer");
+// bc_head_branched, and the serving head of bc_forward_branched_act (mode 0, `actions` may be set, no partials needed)
+static int head_branched_launch(const bc_branched* h, int mode, int64_t* actions, void* stream) {
+    BC_CHECK_ARG(h && h->feat && h->command && h->params && h->out && (h->partials || !(mode & 3)), "bc_head_branched: null buffer");
+    BC_CHECK_ARG(!actions || mode == 0, "bc_head_branched: greedy actions are taken in mode 0 (outputs only)");
     BC_CHECK_ARG(h->n_branches >= 1 && h->n_branches <= 16, "bc_head_branched: n_branches %d outside 1..16", h->n_branches);
     BC_CHECK_ARG(h->n_out >= 1 && h->n_out <= MAXA, "bc_head_branched: n_out %d outside 1..%d", h->n_out, MAXA);
     BC_CHECK_ARG(h->loss_kind >= 0 && h->loss_kind <= 2, "bc_head_branched: loss_kind %d (0 CE, 1 L1, 2 MSE)", h->loss_kind);
@@ -303,12 +317,12 @@ extern "C" int bc_head_branched(const bc_branched* h, int mode, void* stream) {
     if (h->batch == 0 && !(mode & 3)) return BC_OK;
     BrArgs a{};
     a.feat = h->feat; a.cmd = h->command; a.y = h->labels; a.tgt = h->targets; a.params = h->params;
-    a.out = h->out; a.dout = h->dout; a.gfeat = h->gfeat;
+    a.out = h->out; a.dout = h->dout; a.gfeat = h->gfeat; a.actions = actions;
     a.L = head_layout(h->n_out);
     a.B = h->batch; a.NA = h->n_out; a.G = h->n_branches; a.nb = branch_ctas(h->n_branches); a.mode = mode; a.kind = h->loss_kind;
     a.loss_scale = h->loss_scale; a.err = h->err_flag;
     a.part = h->partials;
-    a.loss_part = h->partials + (size_t)a.G * a.nb * a.L.len;
+    a.loss_part = h->partials ? h->partials + (size_t)a.G * a.nb * a.L.len : nullptr;
     bc::launch_pdl(head_branched_kernel, dim3(a.nb, a.G), dim3(NT), 0, (cudaStream_t)stream, a);
     BC_CUDA_LAUNCH_CHECK("head_branched_kernel");
     if (mode & 3) {
@@ -318,4 +332,26 @@ extern "C" int bc_head_branched(const bc_branched* h, int mode, void* stream) {
         BC_CUDA_LAUNCH_CHECK("branched_reduce_kernel");
     }
     return BC_OK;
+}
+
+extern "C" int bc_head_branched(const bc_branched* h, int mode, void* stream) {
+    BC_CHECK_ARG(h && h->partials, "bc_head_branched: null buffer");
+    return head_branched_launch(h, mode, nullptr, stream);
+}
+
+extern "C" int bc_forward_branched_act(const bc_ctx* c, const bc_branched* h, int64_t* actions, int tail, void* stream) {
+    BC_CHECK_ARG(c && h, "bc_forward_branched_act: null ctx / branched heads");
+    BC_CHECK_ARG(h->batch == c->batch, "bc_forward_branched_act: bc_branched.batch %d differs from bc_ctx.batch %d", h->batch, c->batch);
+    BC_CHECK_ARG(!tail || (c->batch >= 0 && c->batch <= BC_POLICY_TAIL_MAX_BATCH),
+                 "bc_forward_branched_act: tail = 1 serves batches up to %d (got %d)", BC_POLICY_TAIL_MAX_BATCH, c->batch);
+    BC_CHECK_ARG(h->params && (uintptr_t)h->params % 16 == 0, "bc_forward_branched_act: the branch arena must be 16 B aligned");
+    BC_CHECK_ARG(c->act[3] || tail, "bc_forward_branched_act: tail = 0 needs act[3] (the heads' features)");
+    for (int l = 0; l < (tail ? 2 : 4); ++l) {
+        int rc = bc_conv_relu_pool_fwd(c, l, stream);
+        if (rc) return rc;
+    }
+    if (tail) return bc_policy_tail_branched(c, h, actions, stream);
+    bc_branched hh = *h;                      // the heads read the trunk's pooled conv4 output
+    hh.feat = c->act[3];
+    return head_branched_launch(&hh, 0, actions, stream);
 }

@@ -21,6 +21,13 @@
 //   phase D  CTA 0: the three Linear layers on all 256 threads (rows split over neighbouring lanes), logits, greedy action
 //            (torch.argmax's rule: the first NaN, else the first maximum).
 // Two cluster barriers per sample; no global-memory round trip between the layers.
+//
+// The branched instantiation (bc_policy_tail_branched) serves ConvNet1Branched: the G heads have the single head's shapes and
+// padded order [fc.4 | fc.2 | fc.0] (head_branched.cu), so the shared-memory plan and phases B..D are the same. Only CTA 0's
+// head load differs: it reads command[b] (before griddepcontrol.wait, like the weights: nothing in this library writes the
+// command vector, include/bc_b200.h launch ordering) and loads branch command[b]'s fc.0, fc.2, fc.4 from the branch arena.
+// A command outside [0, G) loads branch 0 (the address is clamped before any load), raises flag 4 and leaves a zero output
+// row and action 0, as head_branched_kernel does.
 #include "bc_common.cuh"
 #include "trace.cuh"
 #include <cooperative_groups.h>
@@ -72,13 +79,23 @@ struct TailArgs {
     int B, NA;
 };
 
-__global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a) {
+struct BranchArgs {                                     // the branched instantiation only
+    const int64_t* cmd;                                 // (B,) branch ids
+    const float* barena;                                // G x head_len floats, per branch [fc.4 w,b | fc.2 w,b | fc.0 w,b]
+    int64_t head_len, w0, b0, w2, b2, w4, b4;           // bc_head_branched_layout
+    int G;
+    int* err;                                           // flag 4 = command outside [0, G)
+};
+
+template <bool kBranched>
+__global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a, const BranchArgs br) {
     extern __shared__ __align__(16) float sm[];
     cg::cluster_group cluster = cg::this_cluster();
     const int r = (int)cluster.block_rank();
     const int b = blockIdx.x / CL;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int NA = a.NA;
+    bool cmd_ok = true;                  // branched: command[b] in [0, G) (read by CTA 0, which alone writes outputs from it)
     TRACE_T0
     TRACE_DECL
     TRACE(0, 0);
@@ -110,22 +127,29 @@ __global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a) {
         if (tid < 16) sm[O_B4 + tid] = __ldcg(a.b4 + 16 * r + tid);
     }
     if (r == 0) {
-        const float4* w0v = reinterpret_cast<const float4*>(a.f0);
+        const float *f0 = a.f0, *g0 = a.g0, *f2 = a.f2, *g2 = a.g2, *f4 = a.f4, *g4 = a.g4;
+        if constexpr (kBranched) {       // the commanded branch: clamped to branch 0 before any load of its weights
+            const int64_t cmd = __ldcg(br.cmd + b);
+            cmd_ok = cmd >= 0 && cmd < br.G;
+            const float* P = br.barena + (cmd_ok ? cmd : 0) * br.head_len;
+            f0 = P + br.w0; g0 = P + br.b0; f2 = P + br.w2; g2 = P + br.b2; f4 = P + br.w4; g4 = P + br.b4;
+        }
+        const float4* w0v = reinterpret_cast<const float4*>(f0);
         float4 t[8];
 #pragma unroll
         for (int q = 0; q < 8; ++q) t[q] = __ldcg(w0v + tid + NT * q);
-        const float4* w2v = reinterpret_cast<const float4*>(a.f2);
+        const float4* w2v = reinterpret_cast<const float4*>(f2);
         const float4 u0 = __ldcg(w2v + tid), u1 = __ldcg(w2v + tid + NT);
         const bool has4 = tid < NA * 8;
-        const float4 u4 = has4 ? __ldcg(reinterpret_cast<const float4*>(a.f4) + tid) : make_float4(0.f, 0.f, 0.f, 0.f);
+        const float4 u4 = has4 ? __ldcg(reinterpret_cast<const float4*>(f4) + tid) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
         for (int q = 0; q < 8; ++q) reinterpret_cast<float4*>(sm + O_HW0)[tid + NT * q] = t[q];
         reinterpret_cast<float4*>(sm + O_HW2)[tid] = u0;
         reinterpret_cast<float4*>(sm + O_HW2)[tid + NT] = u1;
         if (has4) reinterpret_cast<float4*>(sm + O_HW4)[tid] = u4;
-        if (tid < 64) sm[O_HB0 + tid] = __ldcg(a.g0 + tid);
-        if (tid < 32) sm[O_HB2 + tid] = __ldcg(a.g2 + tid);
-        if (tid < NA) sm[O_HB4 + tid] = __ldcg(a.g4 + tid);
+        if (tid < 64) sm[O_HB0 + tid] = __ldcg(g0 + tid);
+        if (tid < 32) sm[O_HB2 + tid] = __ldcg(g2 + tid);
+        if (tid < NA) sm[O_HB4 + tid] = __ldcg(g4 + tid);
     }
     TRACE(1, 0);
     bc::pdl_wait();                      // act2 is the previous launch's output
@@ -336,15 +360,16 @@ __global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a) {
     __syncthreads();
     if (a.hid1 && tid < 64) a.hid1[(size_t)b * 64 + tid] = s_h1[tid];
     if (a.hid2 && tid < 32) a.hid2[(size_t)b * 32 + tid] = s_h2[tid];
-    if (tid < NA) a.logits[(size_t)b * NA + tid] = s_z[tid];
+    if (tid < NA) a.logits[(size_t)b * NA + tid] = cmd_ok ? s_z[tid] : 0.f;
     if (warp == 0 && a.actions) {
         const float z = lane < NA ? s_z[lane] : -INFINITY;
         const float m = bc::warp_max(z);                                         // fmaxf: drops NaN
         // like torch.argmax: the first NaN if there is one (NaN counts as the maximum), else the first maximum
         const unsigned nan = __ballot_sync(0xffffffffu, lane < NA && isnan(z));
         const unsigned hit = nan ? nan : __ballot_sync(0xffffffffu, lane < NA && z == m);
-        if (lane == 0) a.actions[b] = hit ? (int64_t)(__ffs((int)hit) - 1) : 0;
+        if (lane == 0) a.actions[b] = hit && cmd_ok ? (int64_t)(__ffs((int)hit) - 1) : 0;
     }
+    if (kBranched && !cmd_ok && tid == 0 && br.err) atomicExch(br.err, 4);
     TRACE(9, 0);
     TRACE_END;
 }
@@ -353,17 +378,29 @@ __global__ void __launch_bounds__(NT, 1) policy_tail_kernel(const TailArgs a) {
 
 BC_TRACE_EXPORT(bc_debug_tail_trace)       // debug builds only: not part of the ABI
 
-extern "C" int bc_policy_tail(const bc_ctx* c, int64_t* actions, void* stream) {
-    BC_CHECK_ARG(c && c->params && c->act[1] && c->logits, "bc_policy_tail: null buffer (needs params, act[1], logits)");
-    BC_CHECK_ARG(c->n_actions >= 1 && c->n_actions <= MAXA, "bc_policy_tail: n_actions %d outside 1..%d", c->n_actions, MAXA);
-    BC_CHECK_ARG(c->batch >= 0 && c->batch <= BC_POLICY_TAIL_MAX_BATCH, "bc_policy_tail: batch %d outside 0..%d (one 8-CTA cluster per sample; "
-                 "larger batches belong to the tensor-core kernels: bc_forward_act)", c->batch, BC_POLICY_TAIL_MAX_BATCH);
+// one launcher for both instantiations: `br` NULL = the single head (bc_ctx's fc and logits), else the commanded branch
+static int launch_tail(const bc_ctx* c, const bc_branched* h, int64_t* actions, void* stream) {
+    const char* who = h ? "bc_policy_tail_branched" : "bc_policy_tail";
+    BC_CHECK_ARG(c && c->params && c->act[1], "%s: null buffer (needs params, act[1])", who);
+    BC_CHECK_ARG(c->n_actions >= 1 && c->n_actions <= MAXA, "%s: n_actions %d outside 1..%d", who, c->n_actions, MAXA);
+    BC_CHECK_ARG(c->batch >= 0 && c->batch <= BC_POLICY_TAIL_MAX_BATCH, "%s: batch %d outside 0..%d (one 8-CTA cluster per sample; "
+                 "larger batches belong to the tensor-core kernels: bc_forward_act)", who, c->batch, BC_POLICY_TAIL_MAX_BATCH);
+    if (h) {
+        BC_CHECK_ARG(h->params && h->command && h->out, "%s: null buffer in bc_branched (needs params, command, out)", who);
+        BC_CHECK_ARG(h->n_branches >= 1 && h->n_branches <= 16, "%s: n_branches %d outside 1..16", who, h->n_branches);
+        BC_CHECK_ARG(h->n_out >= 1 && h->n_out <= MAXA, "%s: n_out %d outside 1..%d", who, h->n_out, MAXA);
+        BC_CHECK_ARG(h->batch == c->batch, "%s: bc_branched.batch %d differs from bc_ctx.batch %d", who, h->batch, c->batch);
+        BC_CHECK_ARG((uintptr_t)h->params % 16 == 0, "%s: the branch arena is read as 16 B words", who);
+    } else {
+        BC_CHECK_ARG(c->logits, "%s: null buffer (needs logits)", who);
+    }
     if (c->batch == 0) return BC_OK;
     BC_CHECK_ARG(((uintptr_t)c->params | (uintptr_t)c->act[1]) % 16 == 0 && (!c->act[2] || (uintptr_t)c->act[2] % 16 == 0),
-                 "bc_policy_tail: params, act[1] and act[2] are read / written as 16 B words");
-    static bc::PerDeviceOnce once_; bool& configured = once_();
+                 "%s: params, act[1] and act[2] are read / written as 16 B words", who);
+    void (*kern)(const TailArgs, const BranchArgs) = h ? policy_tail_kernel<true> : policy_tail_kernel<false>;
+    static bc::PerDeviceOnce once_[2]; bool& configured = once_[h ? 1 : 0]();
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(policy_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e != cudaSuccess) return bc::fail(BC_ERR_DEVICE, "policy_tail_kernel: smem opt-in %d B failed: %s", SMEM_BYTES, cudaGetErrorString(e));
         configured = true;
     }
@@ -378,6 +415,15 @@ extern "C" int bc_policy_tail(const bc_ctx* c, int64_t* actions, void* stream) {
     a.act3 = c->act[2]; a.act4 = c->act[3]; a.hid1 = c->hid1; a.hid2 = c->hid2;
     a.logits = c->logits; a.actions = actions;
     a.B = c->batch; a.NA = c->n_actions;
+    BranchArgs br{};
+    if (h) {
+        int64_t off[6], siz[6];                          // state_dict order: 0.weight 0.bias 2.weight 2.bias 4.weight 4.bias
+        br.head_len = bc_head_branched_layout(h->n_out, off, siz);
+        br.w0 = off[0]; br.b0 = off[1]; br.w2 = off[2]; br.b2 = off[3]; br.w4 = off[4]; br.b4 = off[5];
+        br.cmd = h->command; br.barena = h->params; br.G = h->n_branches; br.err = h->err_flag;
+        a.logits = h->out; a.NA = h->n_out;              // fc.0 .. fc.4 come from the branch arena; conv3 / conv4 from the trunk's
+        a.f0 = a.g0 = a.f2 = a.g2 = a.f4 = a.g4 = nullptr;
+    }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(c->batch * CL); cfg.blockDim = dim3(NT); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = (cudaStream_t)stream;
     cudaLaunchAttribute at[2];
@@ -386,8 +432,16 @@ extern "C" int bc_policy_tail(const bc_ctx* c, int64_t* actions, void* stream) {
     at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = 2;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, policy_tail_kernel, a);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a, br);
     if (e != cudaSuccess) bc::pending_launch_error() = e;
     BC_CUDA_LAUNCH_CHECK("policy_tail_kernel");
     return BC_OK;
+}
+
+extern "C" int bc_policy_tail(const bc_ctx* c, int64_t* actions, void* stream) {
+    return launch_tail(c, nullptr, actions, stream);
+}
+
+extern "C" int bc_policy_tail_branched(const bc_ctx* c, const bc_branched* h, int64_t* actions, void* stream) {
+    return launch_tail(c, h, actions, stream);
 }

@@ -72,6 +72,21 @@ def augment_table(seed: int, n_frames: int, src_hw, out_hw=(256, 256), brightnes
     return t
 
 
+def center_crop_table(n_frames: int, src_hw, mean: float = 0.0, std: float = 1.0, out_hw=(256, 256)) -> np.ndarray:
+    """EXTENSION: the deterministic serving counterpart of augment_table -- rows of the same (n_frames, 8) f32 layout with
+    the centre crop ((Hs - 256) // 2, (Ws - 256) // 2), brightness, contrast and saturation factors of exactly 1 and the
+    training normalisation (mean, 1/std). A policy trained on augment_table(..., mean, std) rows is served on these."""
+    if src_hw[0] < out_hw[0] or src_hw[1] < out_hw[1]:
+        raise ValueError(f"source frames {tuple(src_hw)} are smaller than the {out_hw[0]}x{out_hw[1]} crop")
+    t = np.zeros((n_frames, 8), np.float32)
+    t[:, 0] = (src_hw[0] - out_hw[0]) // 2
+    t[:, 1] = (src_hw[1] - out_hw[1]) // 2
+    t[:, 2:5] = 1.0
+    t[:, 5] = mean
+    t[:, 6] = 1.0 / std
+    return t
+
+
 class SequentialFrames:
     """Iterable of (x, y) batches over one frame sequence, staged on the device.
 

@@ -8,6 +8,8 @@ Three layers:
   and what Trainer.fit uses when the module is a ConvNet1-backed Imitation with `cuda_graph: true`.
 * BranchedTrainStep -- the same for the command-conditioned ConvNet1Branched (one GPU): stage [+ augment] -> conv1..4 ->
   branched heads + CE / L1 / MSE -> trunk backward -> Adam on the trunk and the branch arena, one CUDA graph per input slot.
+* BranchedActStep -- its serving counterpart: stage [+ centre crop] -> conv1..4 -> the commanded branches -> greedy action,
+  with the one-launch tail at small batch, one CUDA graph per input slot.
 * Trainer -- epochs over model.train_dataloader() / val_dataloader() with the LightningModule hook order
   (training_step -> zero_grad -> backward -> optimizer.step; validation_step; *_epoch_end; scheduler.step once per epoch
   from training_epoch_end, imitation.py:57-60), ModelCheckpoint(monitor='val_loss', mode='min') in Lightning's .ckpt layout
@@ -128,7 +130,59 @@ class TrainStep:
             self.dp.peer.check()
 
 
-class BranchedTrainStep:
+class _BranchedInput:
+    """The input side BranchedTrainStep and BranchedActStep share: a ConvNet1Branched at a static batch, its staging buffer
+    (f32 planes, or Toeplitz-ready bf16 planes in bf16 mode) and trunk buffers, the checks of frames / table / command, and
+    the staging pass (plain, or crop + jitter + normalise from src_hw sources through a device table)."""
+
+    def _init_input(self, net, batch: int, src_hw, backward: bool) -> None:
+        self.net, self.batch = net, int(batch)
+        if self.batch < 1:
+            raise ValueError("batch must be at least 1")
+        self.src_hw = None if src_hw is None else (int(src_hw[0]), int(src_hw[1]))
+        if self.src_hw is not None and (self.src_hw[0] < 256 or self.src_hw[1] < 256):
+            raise ValueError(f"source frames {self.src_hw} are smaller than the 256x256 crop")
+        self.eng: BCEngine = net.engine()
+        eng, dev, B = self.eng, self.eng.device, self.batch
+        if eng.obs_size != 4:
+            raise ValueError(f"{type(self).__name__} stages 4-frame windows: obs_size must be 4")
+        if not net._barena.is_cuda or net._barena.device != dev:
+            raise RuntimeError("the branch arena must live on the trunk's device (net.to(device))")
+        self.bf16 = bool(eng.conv_mode)
+        if self.bf16:
+            self.staged = StagedBatch(torch.empty((B + 4, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev), None, 4)
+            self.bufs: StepBuffers = eng.alloc(B, self.staged, None, backward)
+        else:
+            self.gray = torch.empty((B + 4, 256, 256), dtype=torch.float32, device=dev)
+            self.bufs = eng.alloc(B, sliding_window(self.gray), None, backward)
+
+    def _check_input(self, frames_u8, table, command) -> None:
+        B, dev = self.batch, self.eng.device
+        hw = self.src_hw or (256, 256)
+        for t, what in ((frames_u8, "frames"), (command, "command")):
+            if not isinstance(t, torch.Tensor) or t.device != dev:
+                raise ValueError(f"{what} must be a tensor on {dev}")
+        if frames_u8.dtype != torch.uint8 or tuple(frames_u8.shape) != (B + 4, *hw, 3) or not frames_u8.is_contiguous():
+            raise ValueError(f"frames must be a contiguous ({B + 4}, {hw[0]}, {hw[1]}, 3) uint8 tensor")
+        if self.src_hw is None:
+            if table is not None:
+                raise ValueError("this step was built without augmentation (src_hw=None): table must be None")
+        elif (not isinstance(table, torch.Tensor) or table.device != dev or table.dtype != torch.float32
+              or tuple(table.shape) != (B + 4, 8) or not table.is_contiguous()):
+            raise ValueError(f"table must be a contiguous ({B + 4}, 8) float32 tensor on {dev} (data.augment_table rows)")
+        if command.dtype != torch.int64 or tuple(command.shape) != (B,) or not command.is_contiguous():
+            raise ValueError(f"command must be a contiguous ({B},) int64 tensor of branch ids")
+
+    def _stage(self, frames_u8, table) -> None:
+        if self.src_hw is not None:
+            stage_augmented(frames_u8, table, layout="tp" if self.bf16 else "plain", out=self.staged if self.bf16 else self.gray)
+        elif self.bf16:
+            stage_frames(frames_u8, out=self.staged)
+        else:
+            stage_gray(frames_u8, out=self.gray)
+
+
+class BranchedTrainStep(_BranchedInput):
     """stage [+ augment] -> conv1..4 -> branched heads + loss + backward -> trunk backward -> Adam on both arenas, for a
     ConvNet1Branched and its MultiArenaAdam at a static batch, captured per input slot like TrainStep.
 
@@ -147,26 +201,10 @@ class BranchedTrainStep:
         if (children is None or len(children) != 2 or children[0]._arena_of is not net
                 or children[1]._arena_of is not net._bowner):
             raise ValueError("BranchedTrainStep takes the net's MultiArenaAdam (net.configure_optimizer())")
-        self.net, self.opt, self.batch, self.graph = net, optimizer, int(batch), graph
+        self.opt, self.graph = optimizer, graph
         self.trunk_opt, self.branch_opt = children
-        if self.batch < 1:
-            raise ValueError("batch must be at least 1")
-        self.src_hw = None if src_hw is None else (int(src_hw[0]), int(src_hw[1]))
-        if self.src_hw is not None and (self.src_hw[0] < 256 or self.src_hw[1] < 256):
-            raise ValueError(f"source frames {self.src_hw} are smaller than the 256x256 crop")
-        self.eng: BCEngine = net.engine()
-        eng, dev, B = self.eng, self.eng.device, self.batch
-        if eng.obs_size != 4:
-            raise ValueError("BranchedTrainStep stages 4-frame windows: obs_size must be 4")
-        if not net._barena.is_cuda or net._barena.device != dev:
-            raise RuntimeError("the branch arena must live on the trunk's device (net.to(device))")
-        self.bf16 = bool(eng.conv_mode)
-        if self.bf16:
-            self.staged = StagedBatch(torch.empty((B + 4, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev), None, 4)
-            self.bufs: StepBuffers = eng.alloc(B, self.staged, None, True)
-        else:
-            self.gray = torch.empty((B + 4, 256, 256), dtype=torch.float32, device=dev)
-            self.bufs = eng.alloc(B, sliding_window(self.gray), None, True)
+        self._init_input(net, batch, src_hw, True)
+        B, dev = self.batch, self.eng.device
         n_part = int(_lib.lib().bc_head_branched_partials_floats(net.n_branches, net.n_actions))
         f32 = dict(dtype=torch.float32, device=dev)
         self.hb = dict(out=torch.empty((B, net.n_actions), **f32), dout=torch.empty((B, net.n_actions), **f32),
@@ -178,33 +216,14 @@ class BranchedTrainStep:
     # ------------------------------------------------------------------ pieces
     def _check_inputs(self, frames_u8, table, command, target) -> None:
         B, dev = self.batch, self.eng.device
-        hw = self.src_hw or (256, 256)
-        for t, what in ((frames_u8, "frames"), (command, "command"), (target, "target")):
-            if not isinstance(t, torch.Tensor) or t.device != dev:
-                raise ValueError(f"{what} must be a tensor on {dev}")
-        if frames_u8.dtype != torch.uint8 or tuple(frames_u8.shape) != (B + 4, *hw, 3) or not frames_u8.is_contiguous():
-            raise ValueError(f"frames must be a contiguous ({B + 4}, {hw[0]}, {hw[1]}, 3) uint8 tensor")
-        if self.src_hw is None:
-            if table is not None:
-                raise ValueError("this step was built without augmentation (src_hw=None): table must be None")
-        elif (not isinstance(table, torch.Tensor) or table.device != dev or table.dtype != torch.float32
-              or tuple(table.shape) != (B + 4, 8) or not table.is_contiguous()):
-            raise ValueError(f"table must be a contiguous ({B + 4}, 8) float32 tensor on {dev} (data.augment_table rows)")
-        if command.dtype != torch.int64 or tuple(command.shape) != (B,) or not command.is_contiguous():
-            raise ValueError(f"command must be a contiguous ({B},) int64 tensor of branch ids")
+        self._check_input(frames_u8, table, command)
+        if not isinstance(target, torch.Tensor) or target.device != dev:
+            raise ValueError(f"target must be a tensor on {dev}")
         if self.net.branch_loss == "ce":
             if target.dtype != torch.int64 or tuple(target.shape) != (B,) or not target.is_contiguous():
                 raise ValueError(f"CE targets are a contiguous ({B},) int64 tensor of class ids")
         elif target.dtype != torch.float32 or tuple(target.shape) != (B, self.net.n_actions) or not target.is_contiguous():
             raise ValueError(f"{self.net.branch_loss} targets are a contiguous ({B}, {self.net.n_actions}) float32 tensor")
-
-    def _stage(self, frames_u8, table) -> None:
-        if self.src_hw is not None:
-            stage_augmented(frames_u8, table, layout="tp" if self.bf16 else "plain", out=self.staged if self.bf16 else self.gray)
-        elif self.bf16:
-            stage_frames(frames_u8, out=self.staged)
-        else:
-            stage_gray(frames_u8, out=self.gray)
 
     def _enqueue(self, frames_u8, table, command, target) -> None:
         self._stage(frames_u8, table)
@@ -243,6 +262,55 @@ class BranchedTrainStep:
 
     def check(self) -> None:
         """Raise if a device-side bounded wait expired, a label (CE) or a command was out of range (synchronises)."""
+        self.eng.check_device_errors()
+
+
+class BranchedActStep(_BranchedInput):
+    """The serving counterpart of BranchedTrainStep: stage [+ centre crop] -> the policy forward of a ConvNet1Branched ->
+    the commanded branches' outputs and, for branch_loss 'ce', the greedy actions, at a static batch, on persistent buffers.
+
+    `act(frames_u8, table, command)`, all on the device: frames (B+4, Hs, Ws, 3) u8; table (B+4, 8) f32 rows when built with
+    src_hw = (Hs, Ws) -- data.center_crop_table(B + 4, src_hw, mean, std) serves a policy trained on augment_table rows --
+    else None; command (B,) int64 branch ids. Returns (out (B, n_out) f32, actions (B,) int64 or None for 'l1' / 'mse'),
+    both persistent, rewritten by the next call. Up to net.tail_batch samples, conv3, conv4 and the head run as one
+    cluster launch (bc_policy_tail_branched). The first call for a given buffer tuple runs eagerly, the second captures a
+    CUDA graph, later calls replay it. The graph holds the command buffer's ADDRESS: the kernels read its contents on
+    every replay, so a caller rewrites it in place per tick (a host copy or a torch op on the stream) and needs no new
+    graph. Nothing in act() synchronises the host; check() does."""
+
+    def __init__(self, net, batch: int, *, src_hw=None, graph: bool = True):
+        self.graph = graph
+        self._init_input(net, batch, src_hw, False)
+        B, dev = self.batch, self.eng.device
+        self.tail = B <= net.tail_batch
+        self.out = torch.empty((B, net.n_actions), dtype=torch.float32, device=dev)
+        self.actions = torch.empty(B, dtype=torch.int64, device=dev) if net.branch_loss == "ce" else None
+        self._seen, self._graphs = set(), {}
+
+    def _enqueue(self, frames_u8, table, command) -> None:
+        self._stage(frames_u8, table)
+        self.net._serve(self.bufs, self.out, self.actions, command, self.tail)
+
+    def act(self, frames_u8: torch.Tensor, table: Optional[torch.Tensor], command: torch.Tensor):
+        """Enqueue one serving forward; returns (out, actions or None)."""
+        self._check_input(frames_u8, table, command)
+        self.eng.ensure_packed()
+        key = (frames_u8.data_ptr(), None if table is None else table.data_ptr(), command.data_ptr())
+        g = self._graphs.get(key) if self.graph else None
+        if g is None and self.graph and key in self._seen:
+            g = self._graphs[key] = torch.cuda.CUDAGraph()
+            with torch.no_grad(), torch.cuda.graph(g):
+                self._enqueue(frames_u8, table, command)
+        if g is not None:
+            g.replay()
+        else:
+            self._seen.add(key)
+            with torch.no_grad():
+                self._enqueue(frames_u8, table, command)
+        return self.out, self.actions
+
+    def check(self) -> None:
+        """Raise if a device-side bounded wait expired or a command was out of range (synchronises)."""
         self.eng.check_device_errors()
 
 

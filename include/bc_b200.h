@@ -156,7 +156,9 @@ int bc_loss_reduce(const bc_ctx* c, void* stream);                 /* head CTAs'
  * optimiser kernels (params, moments, state) -- fetch them BEFORE griddepcontrol.wait, under the previous kernel's tail. That is sound because the kernels that WRITE parameters, moments, state or w_packed (bc_adam_step,
  * bc_adam_tick_step, bc_adam_step_exchange, bc_pack_weights) release their dependents only after their last write. A caller
  * that writes these buffers itself must do so with ordinary (fully serialising) launches or copies -- torch ops are --
- * and never from a kernel of its own that calls griddepcontrol.launch_dependents before its last write. */
+ * and never from a kernel of its own that calls griddepcontrol.launch_dependents before its last write. The same holds for
+ * the command vector of the branched serving tail (bc_policy_tail_branched), which reads command[b] before its wait: no
+ * kernel of this library writes it. */
 
 /* ---- a11: Adam.step (src/models/imitation.py:82-87; torch.optim.Adam defaults).
  * state = 8 DOUBLES {lr, beta1, beta2, eps, step, grad_scale, step_size(out), bc2_sqrt(out)} on the
@@ -243,6 +245,23 @@ typedef struct {
 int bc_head_branched(const bc_branched* h, int mode, void* stream);
 size_t bc_head_branched_partials_floats(int n_branches, int n_out);
 int64_t bc_head_branched_layout(int n_out, int64_t offsets[6], int64_t sizes[6]);
+
+/* ---- K13 for the branched heads: the serving forward of ConvNet1Branched (conditional imitation: the route planner's
+ * command picks the branch per sample, per simulator tick). c = the trunk's context (params, act[], x as for bc_forward_act;
+ * act[2], act[3], hid1, hid2 are written when not NULL), h = the branch arena (params, 16 B aligned), command, out ((batch,
+ * n_out) f32: the commanded branch's outputs) and err_flag; h->feat, labels, targets, grads, dout, gfeat, loss and partials
+ * are not used. h->batch must equal c->batch. actions (batch,) int64 or NULL: the greedy action over out (CE-trained
+ * branches; torch.argmax's rule, K12). A command outside [0, n_branches) sets *err_flag = 4 and leaves a zero out row and
+ * action 0; no branch outside the arena is read.
+ * tail = 0: conv1..conv4, then the branched head kernel (bc_head_branched mode 0) with the action taken inside it.
+ * tail = 1 (batch <= BC_POLICY_TAIL_MAX_BATCH): conv1, conv2, then bc_policy_tail_branched = bc_policy_tail with CTA 0 of
+ *   sample b's cluster loading branch command[b]'s fc.0, fc.2, fc.4 instead of the trunk's fc; same shared memory, same
+ *   arithmetic. The tail reads command[b] BEFORE griddepcontrol.wait, with the weights (launch ordering contract above: no
+ *   kernel of this library writes the command vector; the caller writes it with ordinary stream-ordered work -- a host
+ *   copy, a torch op -- which has completed when the tail starts, because every kernel of this library waits for its
+ *   predecessor before it releases its dependents). */
+int bc_forward_branched_act(const bc_ctx* c, const bc_branched* h, int64_t* actions, int tail, void* stream);
+int bc_policy_tail_branched(const bc_ctx* c, const bc_branched* h, int64_t* actions, void* stream);
 
 /* ---- self-test of the tcgen05/TMEM primitives the bf16 conv kernels are built from:
  * D[M,N] f32 = A[M,K] bf16 * B[N,K]^T bf16 (K contiguous). *err_flag is set to 1 if an mbarrier

@@ -7,6 +7,7 @@ is evaluated, and differentiated, only by branch command[b]) and CE or L1 / MSE 
 
     net = ConvNet1Branched({'obs_size': 4, 'n_actions': 3, 'n_branches': 4, 'branch_loss': 'l1'})
     out = net(x, command)                      # (B, n_out): the commanded branch's outputs
+    act = net.act(x, command)                  # serving: greedy actions (CE) or the branch's controls (L1 / MSE)
     loss = net.loss(x, command, target)        # fused trunk forward + grouped heads + loss; .backward() runs the CUDA backward
 
 The conv trunk is the ConvNet1 arena and kernels unchanged (its single `fc` head stays in the arena, unregistered and
@@ -22,7 +23,7 @@ import torch
 from torch import nn
 
 from carla_imitation_learning_b200 import _lib
-from carla_imitation_learning_b200.engine import _stream_ptr
+from carla_imitation_learning_b200.engine import BCEngine, _stream_ptr, on_device
 from carla_imitation_learning_b200.optim import FusedAdam
 from .nets import ConvNet1, _Slot, _Stack
 
@@ -37,6 +38,12 @@ class _BranchOwner:
 
 
 class ConvNet1Branched(ConvNet1):
+    # serving: up to this batch conv3, conv4 and the commanded branch run as ONE cluster launch (bc_policy_tail_branched),
+    # above it conv3, conv4 and the branched head kernel. Measured crossover (tools/branched_serve_bench.py, B200 at 1000 W,
+    # profiles/r3b_bench_branched_serve.json, p50): tail 22.0-24.0 us against 30.1-32.2 us up to B = 8, 34.24 against
+    # 34.27 at B = 16, 44.5 against 38.4 at B = 32 -- the single head's threshold (BCEngine.tail_batch) again.
+    tail_batch = BCEngine.tail_batch
+
     def __init__(self, hparams):
         super().__init__(hparams)
         self.n_branches = int(hparams['n_branches'])
@@ -176,6 +183,37 @@ class ConvNet1Branched(ConvNet1):
         hb = self._bbufs(x.shape[0])
         self._head(bufs, hb, command, None, 0)
         return hb["out"]
+
+    def _serve(self, bufs, out, actions, command, tail: bool) -> None:
+        """Enqueue the serving forward on the current stream (bc_forward_branched_act): conv1..conv4 and the branched head
+        kernel, or with `tail` conv1, conv2 and the one-launch tail. out (B, n_out) f32 and actions (B,) int64 or None are
+        written; command (B,) int64 is read on the device when the kernels run (a captured graph follows its contents)."""
+        eng = self.engine()
+        c = eng.ctx(bufs)
+        h = _lib.BcBranched()
+        h.n_branches, h.n_out, h.batch, h.loss_kind = self.n_branches, self.n_actions, bufs.batch, LOSS_KINDS[self.branch_loss]
+        h.command, h.params, h.out = command.data_ptr(), self._barena.data_ptr(), out.data_ptr()
+        h.err_flag = eng.err_flag.data_ptr()
+        with on_device(eng.device):
+            _lib.check(eng.lib.bc_forward_branched_act(C.byref(c), C.byref(h), actions.data_ptr() if actions is not None else None,
+                                                       int(bool(tail)), _stream_ptr()), "bc_forward_branched_act")
+
+    @torch.no_grad()
+    def act(self, x, command):
+        """What a conditional-imitation agent sends per tick: for branch_loss 'ce' the (B,) int64 greedy actions of the
+        commanded branches (torch.argmax's rule), for 'l1' / 'mse' their (B, n_out) f32 outputs (steer, throttle, brake).
+        Batches up to `tail_batch` take the one-launch tail. A command outside [0, n_branches)
+        gives a zero row / action 0 and raises at engine().check_device_errors(). For a fixed-shape serving loop use
+        trainer.BranchedActStep (persistent buffers, one CUDA graph per input slot)."""
+        x, command, _ = self._check(x, command, None)
+        eng = self.engine()
+        B = x.shape[0]
+        bufs = eng.alloc(B, x, None, False)
+        out = torch.empty((B, self.n_actions), dtype=torch.float32, device=eng.device)
+        actions = torch.empty(B, dtype=torch.int64, device=eng.device) if self.branch_loss == "ce" else None
+        if B:
+            self._serve(bufs, out, actions, command, B <= self.tail_batch)
+        return actions if actions is not None else out
 
     def loss(self, x, command, target):
         x, command, target = self._check(x, command, target)
