@@ -65,6 +65,8 @@ EXPORTS = {
     "bc_packed_weight_bytes": (C.c_size_t, []),
     "bc_stage_gray_tp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "bc_stage_augment": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "bc_stage_history": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                   C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "bc_planes_to_tp": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "bc_forward": (C.c_int, [C.POINTER(BcCtx), C.c_void_p]),
     "bc_conv_relu_pool_fwd": (C.c_int, [C.POINTER(BcCtx), C.c_int, C.c_void_p]),

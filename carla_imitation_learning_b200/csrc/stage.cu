@@ -25,27 +25,32 @@ __device__ __forceinline__ float gray_px(uint32_t r, uint32_t g, uint32_t b) {
     return __fmaf_rn(rem, rcp, q0);
 }
 
+// gray values of PX consecutive pixels (3 * PX bytes, 4 B aligned)
+template <int PX>
+__device__ __forceinline__ void gray_group(const uint32_t* __restrict__ src, float (&v)[PX]) {
+    uint32_t w[3 * PX / 4];
+#pragma unroll
+    for (int i = 0; i < 3 * PX / 4; ++i) w[i] = __ldg(src + i);
+#pragma unroll
+    for (int p = 0; p < PX; ++p) {
+        uint32_t c[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const int byte = 3 * p + k;
+            c[k] = (w[byte >> 2] >> (8 * (byte & 3))) & 0xffu;
+        }
+        v[p] = gray_px(c[0], c[1], c[2]);
+    }
+}
+
 // PX pixels per thread: 4 for f32 output (one 16 B store), 8 for bf16 output (one 16 B store).
 template <int PX, typename TOUT>
 __global__ void __launch_bounds__(256) stage_gray_kernel(const uint8_t* __restrict__ rgb,
                                                          TOUT* __restrict__ out, int64_t n_groups) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_groups; g += stride) {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(rgb + g * (3 * PX));
-        uint32_t w[3 * PX / 4];
-#pragma unroll
-        for (int i = 0; i < 3 * PX / 4; ++i) w[i] = __ldg(src + i);
         float v[PX];
-#pragma unroll
-        for (int p = 0; p < PX; ++p) {
-            uint32_t c[3];
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                const int byte = 3 * p + k;
-                c[k] = (w[byte >> 2] >> (8 * (byte & 3))) & 0xffu;
-            }
-            v[p] = gray_px(c[0], c[1], c[2]);
-        }
+        gray_group<PX>(reinterpret_cast<const uint32_t*>(rgb + g * (3 * PX)), v);
         if constexpr (sizeof(TOUT) == 4) {
             float4* dst = reinterpret_cast<float4*>(out + g * PX);
 #pragma unroll
@@ -116,6 +121,36 @@ __device__ __forceinline__ float gray_px_bf16_exact(uint32_t px /* bytes R, G, B
     return __fmaf_rn(s, r_lo, __fmul_rn(s, r));
 }
 
+// The 12 gray values of TP unit (R, g') as bf16 pairs: src = the unit's first pixel (4 B aligned); g' = 21 has 4 pixels.
+template <typename I>
+__device__ __forceinline__ void tp_gray_unit(const uint32_t* __restrict__ src, I g, uint32_t (&pk)[6]) {
+    uint32_t w[10];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) w[i] = (g < TP_NG || i < 3) ? __ldg(src + i) : 0u;     // g' = 21 has 4 pixels = 12 bytes left
+    w[9] = 0u;
+    float v[12];
+#pragma unroll
+    for (int p = 0; p < 12; ++p) {
+        constexpr uint32_t sel[4] = {0x1210u, 0x2321u, 0x3432u, 0x4543u};               // bytes o, o+1, o+2, o+1 = R, G, B, G
+        const int o = (3 * p) & 3, i = (3 * p) >> 2;
+        v[p] = gray_px_bf16_exact(__byte_perm(w[i], w[i + 1], sel[o]));
+    }
+#pragma unroll
+    for (int i = 0; i < 6; ++i) pk[i] = pack_bf16(v[2 * i], v[2 * i + 1]);
+}
+
+// Where TP unit (R, g') goes: row0 = the plane's (c = R%3, h = 0, q = R/3) row; pixels 0..7 to segment g' h=0, 8..11 to the
+// first half of its h=1 chunk, 0..3 also to the second half of segment g'-1's h=1 chunk.
+template <typename I>
+__device__ __forceinline__ void tp_store_unit(__nv_bfloat16* row0, I g, const uint32_t (&pk)[6]) {
+    __nv_bfloat16* row1 = row0 + TP_NQ * TP_NG * 8;                                                             // (c, h=1, q)
+    if (g < TP_NG) {
+        *reinterpret_cast<uint4*>(row0 + g * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+        *reinterpret_cast<uint2*>(row1 + g * 8) = make_uint2(pk[4], pk[5]);
+    }
+    if (g > 0) *reinterpret_cast<uint2*>(row1 + (g - 1) * 8 + 4) = make_uint2(pk[0], pk[1]);
+}
+
 __global__ void __launch_bounds__(256) stage_gray_tp_kernel(const uint8_t* __restrict__ rgb, __nv_bfloat16* __restrict__ out,
                                                             __nv_bfloat16* __restrict__ plain, uint32_t n_units) {
     bc::pdl_wait();          // the previous step's kernels still read the planes this one overwrites
@@ -128,33 +163,14 @@ __global__ void __launch_bounds__(256) stage_gray_tp_kernel(const uint8_t* __res
         const uint32_t R = 3u * q + c;
         uint32_t pk[6] = {0, 0, 0, 0, 0, 0};                 // 12 gray values as bf16 pairs; rows R >= 256 stay zero
         if (R < BC_H) {
-            const uint32_t* src = reinterpret_cast<const uint32_t*>(rgb + ((size_t)plane * (BC_H * BC_W) + R * BC_W + 12u * g) * 3);
-            uint32_t w[10];
-#pragma unroll
-            for (int i = 0; i < 9; ++i) w[i] = (g < TP_NG || i < 3) ? __ldg(src + i) : 0u;     // g' = 21 has 4 pixels = 12 bytes left
-            w[9] = 0u;
-            float v[12];
-#pragma unroll
-            for (int p = 0; p < 12; ++p) {
-                constexpr uint32_t sel[4] = {0x1210u, 0x2321u, 0x3432u, 0x4543u};               // bytes o, o+1, o+2, o+1 = R, G, B, G
-                const int o = (3 * p) & 3, i = (3 * p) >> 2;
-                v[p] = gray_px_bf16_exact(__byte_perm(w[i], w[i + 1], sel[o]));
-            }
-#pragma unroll
-            for (int i = 0; i < 6; ++i) pk[i] = pack_bf16(v[2 * i], v[2 * i + 1]);
+            tp_gray_unit(reinterpret_cast<const uint32_t*>(rgb + ((size_t)plane * (BC_H * BC_W) + R * BC_W + 12u * g) * 3), g, pk);
             if (plain) {
                 uint2* dst = reinterpret_cast<uint2*>(plain + ((size_t)plane * BC_H + R) * BC_W + 12u * g);
                 dst[0] = make_uint2(pk[0], pk[1]);
                 if (g < TP_NG) { dst[1] = make_uint2(pk[2], pk[3]); dst[2] = make_uint2(pk[4], pk[5]); }
             }
         }
-        __nv_bfloat16* row0 = out + (size_t)plane * BC_TP_PLANE_ELEMS + ((c * 2u) * TP_NQ + q) * (TP_NG * 8);   // (c, h=0, q)
-        __nv_bfloat16* row1 = row0 + TP_NQ * TP_NG * 8;                                                         // (c, h=1, q)
-        if (g < TP_NG) {
-            *reinterpret_cast<uint4*>(row0 + g * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            *reinterpret_cast<uint2*>(row1 + g * 8) = make_uint2(pk[4], pk[5]);
-        }
-        if (g > 0) *reinterpret_cast<uint2*>(row1 + (g - 1) * 8 + 4) = make_uint2(pk[0], pk[1]);
+        tp_store_unit(out + (size_t)plane * BC_TP_PLANE_ELEMS + ((c * 2u) * TP_NQ + q) * (TP_NG * 8), g, pk);
     }
 }
 
@@ -204,6 +220,20 @@ __device__ __forceinline__ float aug_px(const uint8_t* __restrict__ px, const Au
     return __fmul_rn(__fadd_rn(g, -t.mean), t.istd);
 }
 
+// The 12 augmented values of TP unit (R, g'): src = the unit's first source pixel; g' = 21 has 4 pixels (the rest are 0).
+__device__ __forceinline__ void tp_aug_unit(const uint8_t* __restrict__ src, int g, const AugRow& t, float (&v)[12]) {
+    const int npx = g < TP_NG ? 12 : 4;
+#pragma unroll
+    for (int p = 0; p < 12; ++p) v[p] = p < npx ? aug_px(src + 3 * p, t) : 0.f;
+}
+
+// 4 augmented values of one row: src = the first source pixel
+__device__ __forceinline__ float4 aug4(const uint8_t* __restrict__ src, const AugRow& t) {
+    float4 v;
+    v.x = aug_px(src, t); v.y = aug_px(src + 3, t); v.z = aug_px(src + 6, t); v.w = aug_px(src + 9, t);
+    return v;
+}
+
 // plain f32 planes (n,256,256): one thread = 4 pixels
 __global__ void __launch_bounds__(256) stage_aug_f32_kernel(const uint8_t* __restrict__ rgb, int src_h, int src_w, const AugRow* __restrict__ table,
                                                             float* __restrict__ out, int64_t n_groups) {
@@ -213,9 +243,7 @@ __global__ void __launch_bounds__(256) stage_aug_f32_kernel(const uint8_t* __res
         const int64_t plane = u / ((BC_W / 4) * BC_H);
         const AugRow t = table[plane];
         const uint8_t* src = rgb + ((plane * src_h + (int)t.cy + R) * (int64_t)src_w + (int)t.cx + 4 * x4) * 3;
-        float4 v;
-        v.x = aug_px(src, t); v.y = aug_px(src + 3, t); v.z = aug_px(src + 6, t); v.w = aug_px(src + 9, t);
-        reinterpret_cast<float4*>(out)[u] = v;
+        reinterpret_cast<float4*>(out)[u] = aug4(src, t);
     }
 }
 
@@ -230,21 +258,73 @@ __global__ void __launch_bounds__(256) stage_aug_tp_kernel(const uint8_t* __rest
         uint32_t pk[6] = {0, 0, 0, 0, 0, 0};
         if (R < BC_H) {
             const AugRow t = table[plane];
-            const uint8_t* src = rgb + ((plane * src_h + (int)t.cy + R) * (int64_t)src_w + (int)t.cx + 12 * g) * 3;
-            const int npx = g < TP_NG ? 12 : 4;
             float v[12];
-#pragma unroll
-            for (int p = 0; p < 12; ++p) v[p] = p < npx ? aug_px(src + 3 * p, t) : 0.f;
+            tp_aug_unit(rgb + ((plane * src_h + (int)t.cy + R) * (int64_t)src_w + (int)t.cx + 12 * g) * 3, g, t, v);
 #pragma unroll
             for (int i = 0; i < 6; ++i) pk[i] = pack_bf16(v[2 * i], v[2 * i + 1]);
         }
-        __nv_bfloat16* row0 = out + plane * BC_TP_PLANE_ELEMS + ((int64_t)(c * 2) * TP_NQ + q) * (TP_NG * 8);
-        __nv_bfloat16* row1 = row0 + TP_NQ * TP_NG * 8;
-        if (g < TP_NG) {
-            *reinterpret_cast<uint4*>(row0 + g * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            *reinterpret_cast<uint2*>(row1 + g * 8) = make_uint2(pk[4], pk[5]);
+        tp_store_unit(out + plane * BC_TP_PLANE_ELEMS + ((int64_t)(c * 2) * TP_NQ + q) * (TP_NG * 8), g, pk);
+    }
+}
+
+// ---- EXTENSION: per-agent frame history for closed-loop serving (bc_stage_history). Agent a owns 8 tick slots x `cams` planes,
+// plane (a*8 + j)*cams + k. The frame of tick t goes to slot s = t mod 4 AND s + 4 (every slot on a reset), so the agent's 4-frame
+// window is always the contiguous planes [(s+1)*cams, (s+5)*cams) and conv1 reads it with plain (stride_n, stride_c) =
+// (8*cams, 1) planes. One unit = one destination piece of one frame, converted ONCE by the pixel code of the kernels above and
+// stored 2 (or 8) times. PLANE = elements per plane; TP: one unit of stage_gray_tp_kernel / stage_aug_tp_kernel, else 4 pixels
+// of one row as stage_gray_kernel<4, float> / stage_aug_f32_kernel convert them.
+template <bool TP, bool AUG>
+__global__ void __launch_bounds__(256) stage_history_kernel(const uint8_t* __restrict__ rgb, int src_h, int src_w,
+                                                            const AugRow* __restrict__ table, const uint8_t* __restrict__ reset,
+                                                            int reset_all, void* __restrict__ ring, int cams, int slot,
+                                                            uint32_t n_units) {
+    constexpr uint32_t UPF = TP ? 3u * TP_NQ * TP_NU : (uint32_t)(BC_H * BC_W / 4);     // units per frame
+    constexpr int64_t PLANE = TP ? BC_TP_PLANE_ELEMS : BC_H * BC_W;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t u = blockIdx.x * blockDim.x + threadIdx.x; u < n_units; u += stride) {      // < 2^31: checked on the host
+        const uint32_t row = u / UPF, w = u - row * UPF;             // row = a * cams + k of the frames (and of the table)
+        const uint32_t a = row / (uint32_t)cams, k = row - a * (uint32_t)cams;
+        const bool all = reset_all || (reset != nullptr && reset[a] != 0);
+        int64_t off;                                                  // element offset of this unit inside a plane
+        uint32_t pk[6] = {0, 0, 0, 0, 0, 0};
+        float4 f;
+        uint32_t g = 0;
+        if constexpr (TP) {
+            const uint32_t t1 = w / TP_NU, q = t1 % TP_NQ, c = t1 / TP_NQ, R = 3u * q + c;
+            g = w - t1 * TP_NU;
+            off = (int64_t)((c * 2u) * TP_NQ + q) * (TP_NG * 8);
+            if (R < BC_H) {
+                if constexpr (AUG) {
+                    const AugRow t = table[row];
+                    float v[12];
+                    tp_aug_unit(rgb + (((int64_t)row * src_h + (int)t.cy + (int)R) * (int64_t)src_w + (int)t.cx + 12 * (int)g) * 3, (int)g, t, v);
+#pragma unroll
+                    for (int i = 0; i < 6; ++i) pk[i] = pack_bf16(v[2 * i], v[2 * i + 1]);
+                } else {
+                    tp_gray_unit(reinterpret_cast<const uint32_t*>(rgb + ((size_t)row * (BC_H * BC_W) + R * BC_W + 12u * g) * 3), g, pk);
+                }
+            }
+        } else {
+            off = (int64_t)w * 4;
+            if constexpr (AUG) {
+                const AugRow t = table[row];
+                const int R = (int)(w / (BC_W / 4)), x4 = (int)(w % (BC_W / 4));
+                f = aug4(rgb + (((int64_t)row * src_h + (int)t.cy + R) * (int64_t)src_w + (int)t.cx + 4 * x4) * 3, t);
+            } else {
+                float v[4];
+                gray_group<4>(reinterpret_cast<const uint32_t*>(rgb + ((size_t)row * (BC_H * BC_W) + 4u * w) * 3), v);
+                f = make_float4(v[0], v[1], v[2], v[3]);
+            }
         }
-        if (g > 0) *reinterpret_cast<uint2*>(row1 + (g - 1) * 8 + 4) = make_uint2(pk[0], pk[1]);
+        bc::pdl_wait();      // the previous tick's conv1 may still read the slot this unit overwrites
+        bc::pdl_trigger();
+        for (int j = all ? 0 : slot; j < 8; j += all ? 1 : 4) {
+            const int64_t plane = ((int64_t)a * 8 + j) * cams + k;   // 64-bit: 4096 agents x 3 cameras x 8 slots of TP planes ~ 8.5e9 elements
+            if constexpr (TP)
+                tp_store_unit(reinterpret_cast<__nv_bfloat16*>(ring) + plane * PLANE + off, g, pk);
+            else
+                *reinterpret_cast<float4*>(reinterpret_cast<float*>(ring) + plane * PLANE + off) = f;
+        }
     }
 }
 
@@ -325,5 +405,35 @@ extern "C" int bc_stage_gray(const uint8_t* rgb, void* gray, int64_t n_pixels, i
         stage_gray_kernel<8, __nv_bfloat16><<<blocks, 256, 0, s>>>(rgb, (__nv_bfloat16*)gray, groups);
     }
     BC_CUDA_LAUNCH_CHECK("stage_gray_kernel");
+    return BC_OK;
+}
+
+extern "C" int bc_stage_history(const uint8_t* rgb, int n_agents, int cams, int src_h, int src_w, const float* table,
+                                const uint8_t* reset, int reset_all, void* ring, int slot, int out_dtype, void* stream) {
+    BC_CHECK_ARG(rgb && ring, "bc_stage_history: null pointer (rgb, ring)");
+    BC_CHECK_ARG(n_agents >= 1, "bc_stage_history: n_agents=%d must be at least 1", n_agents);
+    BC_CHECK_ARG(cams == 1 || cams == 3, "bc_stage_history: cams=%d must be 1 or 3 (obs_size 4 or 12)", cams);
+    BC_CHECK_ARG(slot >= 0 && slot < 4, "bc_stage_history: slot=%d must lie in [0, 4) (tick mod 4)", slot);
+    BC_CHECK_ARG(src_h >= BC_H && src_w >= BC_W, "bc_stage_history: source frames %dx%d are smaller than %dx%d", src_h, src_w, BC_H, BC_W);
+    BC_CHECK_ARG(table || (src_h == BC_H && src_w == BC_W), "bc_stage_history: %dx%d sources need a crop table", src_h, src_w);
+    BC_CHECK_ARG(out_dtype == BC_F32 || out_dtype == BC_BF16_TP, "bc_stage_history: the ring holds BC_F32 or BC_BF16_TP planes, got %d", out_dtype);
+    BC_CHECK_ARG((uintptr_t)ring % 16 == 0 && (uintptr_t)table % 16 == 0, "bc_stage_history: ring and table must be 16 B aligned");
+    BC_CHECK_ARG(table || (uintptr_t)rgb % 4 == 0, "bc_stage_history: rgb must be 4 B aligned");
+    const bool tp = out_dtype == BC_BF16_TP;
+    const int64_t units = (int64_t)n_agents * cams * (tp ? 3 * TP_NQ * TP_NU : BC_H * BC_W / 4);
+    BC_CHECK_ARG(units < (int64_t)0x7fffffff - 0x1000000, "bc_stage_history: %d agents x %d cameras in one call (32-bit unit index)", n_agents, cams);
+    const int64_t cap = (int64_t)bc::num_sms() * 16;
+    const int blocks = (int)((units + 255) / 256 < cap ? (units + 255) / 256 : cap);
+    const AugRow* t = (const AugRow*)table;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tp && table)
+        bc::launch_pdl(stage_history_kernel<true, true>, dim3(blocks), dim3(256), 0, s, rgb, src_h, src_w, t, reset, reset_all, ring, cams, slot, (uint32_t)units);
+    else if (tp)
+        bc::launch_pdl(stage_history_kernel<true, false>, dim3(blocks), dim3(256), 0, s, rgb, src_h, src_w, t, reset, reset_all, ring, cams, slot, (uint32_t)units);
+    else if (table)
+        bc::launch_pdl(stage_history_kernel<false, true>, dim3(blocks), dim3(256), 0, s, rgb, src_h, src_w, t, reset, reset_all, ring, cams, slot, (uint32_t)units);
+    else
+        bc::launch_pdl(stage_history_kernel<false, false>, dim3(blocks), dim3(256), 0, s, rgb, src_h, src_w, t, reset, reset_all, ring, cams, slot, (uint32_t)units);
+    BC_CUDA_LAUNCH_CHECK("stage_history_kernel");
     return BC_OK;
 }

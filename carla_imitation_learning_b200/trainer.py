@@ -10,6 +10,8 @@ Three layers:
   branched heads + CE / L1 / MSE -> trunk backward -> Adam on the trunk and the branch arena, one CUDA graph per input slot.
 * BranchedActStep -- its serving counterpart: stage [+ centre crop] -> conv1..4 -> the commanded branches -> greedy action,
   with the one-launch tail at small batch, one CUDA graph per input slot.
+* RolloutActStep -- serving N independent agents per tick: one new frame per agent staged into its on-device history,
+  each agent's window read in place, single head or branched, one CUDA graph per input slot and tick slot.
 * Trainer -- epochs over model.train_dataloader() / val_dataloader() with the LightningModule hook order
   (training_step -> zero_grad -> backward -> optimizer.step; validation_step; *_epoch_end; scheduler.step once per epoch
   from training_epoch_end, imitation.py:57-60), ModelCheckpoint(monitor='val_loss', mode='min') in Lightning's .ckpt layout
@@ -18,6 +20,7 @@ Three layers:
 """
 from __future__ import annotations
 
+import ctypes as C
 import os
 from typing import Callable, Dict, List, Optional
 
@@ -25,7 +28,8 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .engine import BCEngine, StagedBatch, StepBuffers, stage_augmented, stage_frames, stage_gray, sliding_window
+from .engine import (BCEngine, StagedBatch, StepBuffers, _stream_ptr, on_device, stage_augmented, stage_frames, stage_gray,
+                     sliding_window)
 from .optim import FusedAdam
 
 
@@ -131,11 +135,11 @@ class TrainStep:
 
 
 class _BranchedInput:
-    """The input side BranchedTrainStep and BranchedActStep share: a ConvNet1Branched at a static batch, its staging buffer
-    (f32 planes, or Toeplitz-ready bf16 planes in bf16 mode) and trunk buffers, the checks of frames / table / command, and
-    the staging pass (plain, or crop + jitter + normalise from src_hw sources through a device table)."""
+    """The input side BranchedTrainStep, BranchedActStep and RolloutActStep share: a ConvNet1Branched at a static batch, its
+    staging buffer (f32 planes, or Toeplitz-ready bf16 planes in bf16 mode) and trunk buffers, the checks of frames / table /
+    command, and the staging pass (plain, or crop + jitter + normalise from src_hw sources through a device table)."""
 
-    def _init_input(self, net, batch: int, src_hw, backward: bool) -> None:
+    def _init_net(self, net, batch: int, src_hw) -> None:
         self.net, self.batch = net, int(batch)
         if self.batch < 1:
             raise ValueError("batch must be at least 1")
@@ -143,12 +147,18 @@ class _BranchedInput:
         if self.src_hw is not None and (self.src_hw[0] < 256 or self.src_hw[1] < 256):
             raise ValueError(f"source frames {self.src_hw} are smaller than the 256x256 crop")
         self.eng: BCEngine = net.engine()
-        eng, dev, B = self.eng, self.eng.device, self.batch
-        if eng.obs_size != 4:
+        self.bf16 = bool(self.eng.conv_mode)
+
+    def _check_branched_net(self, net) -> None:
+        if self.eng.obs_size != 4:
             raise ValueError(f"{type(self).__name__} stages 4-frame windows: obs_size must be 4")
-        if not net._barena.is_cuda or net._barena.device != dev:
+        if not net._barena.is_cuda or net._barena.device != self.eng.device:
             raise RuntimeError("the branch arena must live on the trunk's device (net.to(device))")
-        self.bf16 = bool(eng.conv_mode)
+
+    def _init_input(self, net, batch: int, src_hw, backward: bool) -> None:
+        self._init_net(net, batch, src_hw)
+        self._check_branched_net(net)
+        eng, dev, B = self.eng, self.eng.device, self.batch
         if self.bf16:
             self.staged = StagedBatch(torch.empty((B + 4, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev), None, 4)
             self.bufs: StepBuffers = eng.alloc(B, self.staged, None, backward)
@@ -157,19 +167,27 @@ class _BranchedInput:
             self.bufs = eng.alloc(B, sliding_window(self.gray), None, backward)
 
     def _check_input(self, frames_u8, table, command) -> None:
-        B, dev = self.batch, self.eng.device
+        self._check_frames(frames_u8, table, self.batch + 4)
+        self._check_command(command)
+
+    def _check_frames(self, frames_u8, table, rows: int) -> None:
+        dev = self.eng.device
         hw = self.src_hw or (256, 256)
-        for t, what in ((frames_u8, "frames"), (command, "command")):
-            if not isinstance(t, torch.Tensor) or t.device != dev:
-                raise ValueError(f"{what} must be a tensor on {dev}")
-        if frames_u8.dtype != torch.uint8 or tuple(frames_u8.shape) != (B + 4, *hw, 3) or not frames_u8.is_contiguous():
-            raise ValueError(f"frames must be a contiguous ({B + 4}, {hw[0]}, {hw[1]}, 3) uint8 tensor")
+        if not isinstance(frames_u8, torch.Tensor) or frames_u8.device != dev:
+            raise ValueError(f"frames must be a tensor on {dev}")
+        if frames_u8.dtype != torch.uint8 or tuple(frames_u8.shape) != (rows, *hw, 3) or not frames_u8.is_contiguous():
+            raise ValueError(f"frames must be a contiguous ({rows}, {hw[0]}, {hw[1]}, 3) uint8 tensor")
         if self.src_hw is None:
             if table is not None:
                 raise ValueError("this step was built without augmentation (src_hw=None): table must be None")
         elif (not isinstance(table, torch.Tensor) or table.device != dev or table.dtype != torch.float32
-              or tuple(table.shape) != (B + 4, 8) or not table.is_contiguous()):
-            raise ValueError(f"table must be a contiguous ({B + 4}, 8) float32 tensor on {dev} (data.augment_table rows)")
+              or tuple(table.shape) != (rows, 8) or not table.is_contiguous()):
+            raise ValueError(f"table must be a contiguous ({rows}, 8) float32 tensor on {dev} (data.augment_table rows)")
+
+    def _check_command(self, command) -> None:
+        B, dev = self.batch, self.eng.device
+        if not isinstance(command, torch.Tensor) or command.device != dev:
+            raise ValueError(f"command must be a tensor on {dev}")
         if command.dtype != torch.int64 or tuple(command.shape) != (B,) or not command.is_contiguous():
             raise ValueError(f"command must be a contiguous ({B},) int64 tensor of branch ids")
 
@@ -307,6 +325,124 @@ class BranchedActStep(_BranchedInput):
             self._seen.add(key)
             with torch.no_grad():
                 self._enqueue(frames_u8, table, command)
+        return self.out, self.actions
+
+    def check(self) -> None:
+        """Raise if a device-side bounded wait expired or a command was out of range (synchronises)."""
+        self.eng.check_device_errors()
+
+
+class RolloutActStep(_BranchedInput):
+    """Closed-loop serving of N independent agents: each agent has its own frame stream, and its frame history lives on the
+    device. Serves a ConvNet1 (obs_size 4 or 12) or a ConvNet1Branched (obs_size 4), fp32 or bf16.
+
+    `act(frames_u8, reset, table=None, command=None)`, all on the device, once per tick: frames (N*cams, Hs, Ws, 3) u8 with
+    cams = obs_size / 4, row a*cams + k = camera k of agent a at this tick; reset (N,) bool or uint8, nonzero = agent a
+    starts a new episode with this frame; table (N*cams, 8) f32 rows when built with src_hw = (Hs, Ws)
+    (data.center_crop_table), else None; command (N,) int64 branch ids for the branched net only. Returns persistent
+    buffers, rewritten by the next tick: (logits (N, n_actions), actions (N,) int64) for the single head, (out (N, n_out),
+    actions or None) for the branched net, as BranchedActStep returns.
+
+    Hidden state: every agent owns 8 tick slots of staged planes (bc_stage_history). One tick stages ONE new frame per
+    agent and camera; the agent's 4-frame window is read in place by conv1, oldest frame first. All agents advance in
+    lockstep: one frame per agent per tick. An agent whose episode has ended is reset with its next episode's first frame
+    (its window is then that frame four times, and the frames that follow push it out one per tick), or its output is
+    ignored. The first tick after construction, and the first after reset_all(), resets every agent whatever `reset` says.
+
+    Up to net.tail_batch agents, conv3, conv4 and the head run as one cluster launch, as on the other serving paths. The
+    slot (tick mod 4) is host state and selects the window, so there is one CUDA graph per (input buffer tuple, slot):
+    the first call for a key runs eagerly, the second captures, later calls replay. The frames, reset, table and command
+    buffers are read on every replay, so a caller rewrites them in place per tick. Nothing in act() synchronises the host;
+    check() does."""
+
+    def __init__(self, net, n_agents: int, *, src_hw=None, graph: bool = True):
+        self.graph = graph
+        self._init_net(net, n_agents, src_hw)
+        eng, dev, N = self.eng, self.eng.device, self.batch
+        self.branched = hasattr(net, "_barena")
+        if self.branched:
+            self._check_branched_net(net)
+        self.cams = eng.obs_size // 4
+        rows = N * 8 * self.cams
+        if self.bf16:
+            self.ring = torch.empty((rows, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev)
+            self.bufs: StepBuffers = eng.alloc(N, StagedBatch(self.ring, None, eng.obs_size, self.cams), None, False)
+        else:
+            self.ring = torch.empty((rows, 256, 256), dtype=torch.float32, device=dev)
+            self.bufs = eng.alloc(N, self._window(0), None, False)
+        self.tail = N <= (net.tail_batch if self.branched else eng.tail_batch)
+        self.actions = torch.empty(N, dtype=torch.int64, device=dev)
+        if self.branched:
+            self.out = torch.empty((N, net.n_actions), dtype=torch.float32, device=dev)
+            if net.branch_loss != "ce":
+                self.actions = None
+        else:
+            self.out = self.bufs.logits
+        self._tick, self._all = 0, True
+        self._seen, self._graphs = set(), {}
+
+    def _window(self, slot: int) -> torch.Tensor:
+        """fp32: the (N, obs, 256, 256) view of every agent's window at `slot`: planes [(slot+1)*cams, (slot+5)*cams)."""
+        P = 256 * 256
+        return self.ring.as_strided((self.batch, self.eng.obs_size, 256, 256), (8 * self.cams * P, P, 256, 1),
+                                    self.ring.storage_offset() + (slot + 1) * self.cams * P)
+
+    def _point(self, slot: int) -> None:
+        if self.bf16:
+            E = _lib.TP_PLANE_ELEMS
+            self.bufs.x_tp, self.bufs.x_tp_strides = self.ring[(slot + 1) * self.cams:], (8 * self.cams * E, E)
+        else:
+            self.bufs.x = self._window(slot)
+
+    def reset_all(self) -> None:
+        """The next tick starts a new episode for every agent."""
+        self._all = True
+
+    def _enqueue(self, frames_u8, reset, table, command, slot: int, reset_all: bool) -> None:
+        eng = self.eng
+        self._point(slot)
+        hs, ws = frames_u8.shape[1], frames_u8.shape[2]
+        with on_device(eng.device):
+            _lib.check(eng.lib.bc_stage_history(frames_u8.data_ptr(), self.batch, self.cams, hs, ws,
+                                                None if table is None else table.data_ptr(), reset.data_ptr(),
+                                                int(reset_all), self.ring.data_ptr(), slot,
+                                                _lib.BC_BF16_TP if self.bf16 else _lib.BC_F32, _stream_ptr()),
+                       "bc_stage_history")
+            if self.branched:
+                self.net._serve(self.bufs, self.out, self.actions, command, self.tail)
+            else:
+                c = eng.ctx(self.bufs)
+                _lib.check(eng.lib.bc_forward_act(C.byref(c), self.actions.data_ptr(), int(self.tail), _stream_ptr()),
+                           "bc_forward_act")
+
+    def act(self, frames_u8: torch.Tensor, reset: torch.Tensor, table: Optional[torch.Tensor] = None,
+            command: Optional[torch.Tensor] = None):
+        """Enqueue one tick: stage each agent's new frame into its history, then serve every agent's window."""
+        self._check_frames(frames_u8, table, self.batch * self.cams)
+        dev = self.eng.device
+        if (not isinstance(reset, torch.Tensor) or reset.device != dev or reset.dtype not in (torch.bool, torch.uint8)
+                or tuple(reset.shape) != (self.batch,) or not reset.is_contiguous()):
+            raise ValueError(f"reset must be a contiguous ({self.batch},) bool or uint8 tensor on {dev}")
+        if self.branched:
+            self._check_command(command)
+        elif command is not None:
+            raise ValueError("a single-head ConvNet1 takes no command (command must be None)")
+        self.eng.ensure_packed()
+        slot, everyone = self._tick % 4, self._all
+        key = (frames_u8.data_ptr(), reset.data_ptr(), None if table is None else table.data_ptr(),
+               None if command is None else command.data_ptr(), slot, everyone)
+        g = self._graphs.get(key) if self.graph else None
+        if g is None and self.graph and key in self._seen:
+            g = self._graphs[key] = torch.cuda.CUDAGraph()
+            with torch.no_grad(), torch.cuda.graph(g):
+                self._enqueue(frames_u8, reset, table, command, slot, everyone)
+        if g is not None:
+            g.replay()
+        else:
+            self._seen.add(key)
+            with torch.no_grad():
+                self._enqueue(frames_u8, reset, table, command, slot, everyone)
+        self._tick, self._all = self._tick + 1, False
         return self.out, self.actions
 
     def check(self) -> None:

@@ -112,6 +112,24 @@ int bc_stage_gray_tp(const uint8_t* rgb, void* tp, void* plain_bf16, int64_t n_f
  * f32 rounding; the un-augmented kernels stay the bit-exact ones. */
 int bc_stage_augment(const uint8_t* rgb, int64_t n_frames, int src_h, int src_w, const float* table, void* out, int out_dtype, void* stream);
 
+/* EXTENSION: the per-agent frame history of closed-loop serving (N agents, each with its own frame stream, advancing one frame
+ * per tick in lockstep). ring = n_agents x 8 tick slots x cams planes (cams = obs_size / 4: 1 or 3), plane (a*8 + j)*cams + k,
+ * each plane BC_F32 (256x256 f32) or BC_BF16_TP (BC_TP_PLANE_ELEMS bf16); 64-bit addressing (4096 x 3 x 8 TP planes ~ 17 GB).
+ * rgb (n_agents*cams, src_h, src_w, 3) u8, row a*cams + k = camera k of agent a at this tick. slot = tick mod 4: the frame is
+ * written to slots `slot` AND `slot + 4`, so the agent's window is the contiguous planes [(slot+1)*cams, (slot+5)*cams) of its
+ * ring, oldest frame first, channel = cams*frame + camera (the order of sliding_window(step=3)): conv1 reads it with
+ * x (or x_tp) = ring + (slot+1)*cams planes, stride_c = 1 plane, stride_n = 8*cams planes.
+ * An agent with reset[a] != 0 (reset: (n_agents,) u8 or NULL), or every agent when reset_all, gets the frame in all 8 slots:
+ * its window is the first frame four times (the frame-stack convention at an episode start). No other plane is written.
+ * table NULL (256x256 sources only): every written plane is bitwise what bc_stage_gray(BC_F32) / bc_stage_gray_tp writes for
+ * that frame; table ((n_agents*cams, 8) f32 rows, 16 B aligned): bitwise what bc_stage_augment writes for that frame and row
+ * (data.center_crop_table serves a policy trained on augment_table rows). Arguments are checked before any CUDA call:
+ * n_agents >= 1, cams in {1, 3}, slot in [0, 4), src >= 256, ring and table 16 B aligned. Launched with programmatic stream
+ * serialisation; the kernel waits for its predecessor before its first store (the previous tick's conv1 reads the slot it
+ * overwrites) and may read rgb, table and reset before that wait (launch-ordering contract below). */
+int bc_stage_history(const uint8_t* rgb, int n_agents, int cams, int src_h, int src_w, const float* table,
+                     const uint8_t* reset, int reset_all, void* ring, int slot, int out_dtype, void* stream);
+
 /* plain planes (f32 or bf16; 256x256, rows contiguous, `plane_stride` elements apart) -> BC_BF16_TP planes:
  * how a reference-style (B,4,256,256) batch enters the tcgen05 conv1 (bf16 mode) */
 int bc_planes_to_tp(const void* planes, int in_dtype, int64_t n_planes, int64_t plane_stride, void* out_tp, void* stream);
@@ -158,7 +176,8 @@ int bc_loss_reduce(const bc_ctx* c, void* stream);                 /* head CTAs'
  * that writes these buffers itself must do so with ordinary (fully serialising) launches or copies -- torch ops are --
  * and never from a kernel of its own that calls griddepcontrol.launch_dependents before its last write. The same holds for
  * the command vector of the branched serving tail (bc_policy_tail_branched), which reads command[b] before its wait: no
- * kernel of this library writes it. */
+ * kernel of this library writes it. No kernel of this library writes the reset vector of bc_stage_history either: the caller
+ * writes it with stream-ordered work, as it does the command vector. */
 
 /* ---- a11: Adam.step (src/models/imitation.py:82-87; torch.optim.Adam defaults).
  * state = 8 DOUBLES {lr, beta1, beta2, eps, step, grad_scale, step_size(out), bc2_sqrt(out)} on the
