@@ -56,6 +56,13 @@ class BcBranched(C.Structure):
                 ("loss_scale", C.c_float)]
 
 
+class BcFrameStore(C.Structure):
+    """Mirror of `bc_frame_store` (include/bc_b200.h): a frame store in device memory for bc_stage_gather."""
+    _fields_ = [("frames", C.c_void_p), ("n_frames", C.c_int64), ("cams", C.c_int32), ("src_h", C.c_int32),
+                ("src_w", C.c_int32), ("labels", C.c_void_p), ("commands", C.c_void_p), ("targets", C.c_void_p),
+                ("n_out", C.c_int32)]
+
+
 EXPORTS = {
     # name: (restype, argtypes)
     "bc_arena_layout": (C.c_int64, [C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
@@ -67,6 +74,8 @@ EXPORTS = {
     "bc_stage_augment": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "bc_stage_history": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                    C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "bc_stage_gather": (C.c_int, [C.POINTER(BcFrameStore), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bc_planes_to_tp": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "bc_forward": (C.c_int, [C.POINTER(BcCtx), C.c_void_p]),
     "bc_conv_relu_pool_fwd": (C.c_int, [C.POINTER(BcCtx), C.c_int, C.c_void_p]),

@@ -328,6 +328,81 @@ __global__ void __launch_bounds__(256) stage_history_kernel(const uint8_t* __res
     }
 }
 
+// ---- EXTENSION: shuffled minibatches from a device-resident frame store (bc_stage_gather). Sample b is the reference's sample
+// i = index[b]: frames i .. i+3, side data of frame i+4. Output plane b*4*cams + cams*j + k = camera k of frame i+j (the channel
+// order of sliding_window(step=cams), materialised). One unit = one piece of one output plane, in the unit decomposition of
+// stage_history_kernel and converted by the same pixel code; every unit is stored once. A sample whose index lies outside
+// [0, n_frames - 5] reads nothing and gets zero planes, zero side data and err_flag 5.
+template <bool TP, bool AUG>
+__global__ void __launch_bounds__(256) stage_gather_kernel(bc_frame_store s, const int64_t* __restrict__ index, int batch,
+                                                           const AugRow* __restrict__ table, void* __restrict__ out,
+                                                           int64_t* __restrict__ y, int64_t* __restrict__ command,
+                                                           float* __restrict__ target, int32_t* __restrict__ err_flag,
+                                                           uint32_t n_units) {
+    constexpr uint32_t UPF = TP ? 3u * TP_NQ * TP_NU : (uint32_t)(BC_H * BC_W / 4);     // units per plane
+    constexpr int64_t PLANE = TP ? BC_TP_PLANE_ELEMS : BC_H * BC_W;
+    const uint32_t cams = (uint32_t)s.cams, pps = 4u * cams;                             // planes per sample
+    const int64_t last = s.n_frames - 5;
+    const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;
+    for (uint32_t u = tid; u < n_units; u += stride) {                // < 2^31: checked on the host
+        const uint32_t p = u / UPF, w = u - p * UPF;                  // output plane p
+        const uint32_t b = p / pps, r = p - b * pps, j = r / cams, k = r - j * cams;
+        const int64_t i = __ldg(index + b);
+        const bool ok = i >= 0 && i <= last;
+        const int64_t row = (i + j) * cams + k;                       // store row (64-bit: a store is tens of GB)
+        int64_t off;
+        uint32_t pk[6] = {0, 0, 0, 0, 0, 0};
+        float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
+        uint32_t g = 0;
+        if constexpr (TP) {
+            const uint32_t t1 = w / TP_NU, q = t1 % TP_NQ, c = t1 / TP_NQ, R = 3u * q + c;
+            g = w - t1 * TP_NU;
+            off = (int64_t)((c * 2u) * TP_NQ + q) * (TP_NG * 8);
+            if (ok && R < BC_H) {
+                if constexpr (AUG) {
+                    const AugRow t = table[b * cams + k];
+                    float v[12];
+                    tp_aug_unit(s.frames + ((row * s.src_h + (int)t.cy + (int)R) * (int64_t)s.src_w + (int)t.cx + 12 * (int)g) * 3, (int)g, t, v);
+#pragma unroll
+                    for (int m = 0; m < 6; ++m) pk[m] = pack_bf16(v[2 * m], v[2 * m + 1]);
+                } else {
+                    tp_gray_unit(reinterpret_cast<const uint32_t*>(s.frames + (row * (BC_H * BC_W) + R * BC_W + 12u * g) * 3), g, pk);
+                }
+            }
+        } else {
+            off = (int64_t)w * 4;
+            if (ok) {
+                if constexpr (AUG) {
+                    const AugRow t = table[b * cams + k];
+                    const int R = (int)(w / (BC_W / 4)), x4 = (int)(w % (BC_W / 4));
+                    f = aug4(s.frames + ((row * s.src_h + (int)t.cy + R) * (int64_t)s.src_w + (int)t.cx + 4 * x4) * 3, t);
+                } else {
+                    float v[4];
+                    gray_group<4>(reinterpret_cast<const uint32_t*>(s.frames + (row * (BC_H * BC_W) + 4u * w) * 3), v);
+                    f = make_float4(v[0], v[1], v[2], v[3]);
+                }
+            }
+        }
+        bc::pdl_wait();      // the previous step's conv1 (forward and weight gradient) may still read the planes this unit overwrites
+        bc::pdl_trigger();
+        if constexpr (TP)
+            tp_store_unit(reinterpret_cast<__nv_bfloat16*>(out) + (int64_t)p * PLANE + off, g, pk);
+        else
+            *reinterpret_cast<float4*>(reinterpret_cast<float*>(out) + (int64_t)p * PLANE + off) = f;
+    }
+    // side data of frame i+4, in the same launch: the previous step's head may still read these buffers
+    bc::pdl_wait();
+    for (uint32_t b = tid; b < (uint32_t)batch; b += stride) {
+        const int64_t i = __ldg(index + b);
+        const bool ok = i >= 0 && i <= last;
+        if (!ok) atomicCAS(err_flag, 0, 5);                        // never masks an error code already set
+        if (y && s.labels) y[b] = ok ? __ldg(s.labels + i + 4) : 0;
+        if (command && s.commands) command[b] = ok ? __ldg(s.commands + i + 4) : 0;
+        if (target && s.targets)
+            for (int o = 0; o < s.n_out; ++o) target[(int64_t)b * s.n_out + o] = ok ? __ldg(s.targets + (i + 4) * s.n_out + o) : 0.f;
+    }
+}
+
 }  // namespace
 
 extern "C" int bc_stage_augment(const uint8_t* rgb, int64_t n_frames, int src_h, int src_w, const float* table, void* out, int out_dtype, void* stream) {
@@ -435,5 +510,39 @@ extern "C" int bc_stage_history(const uint8_t* rgb, int n_agents, int cams, int 
     else
         bc::launch_pdl(stage_history_kernel<false, false>, dim3(blocks), dim3(256), 0, s, rgb, src_h, src_w, t, reset, reset_all, ring, cams, slot, (uint32_t)units);
     BC_CUDA_LAUNCH_CHECK("stage_history_kernel");
+    return BC_OK;
+}
+
+extern "C" int bc_stage_gather(const bc_frame_store* st, const int64_t* index, int batch, const float* table, void* out,
+                               int out_dtype, int64_t* y, int64_t* command, float* target, int32_t* err_flag, void* stream) {
+    BC_CHECK_ARG(st && st->frames && index && out && err_flag, "bc_stage_gather: null pointer (store, frames, index, out, err_flag)");
+    BC_CHECK_ARG(batch >= 1, "bc_stage_gather: batch=%d must be at least 1", batch);
+    BC_CHECK_ARG(st->cams == 1 || st->cams == 3, "bc_stage_gather: cams=%d must be 1 or 3 (obs_size 4 or 12)", st->cams);
+    BC_CHECK_ARG(st->n_frames >= 5, "bc_stage_gather: n_frames=%lld: a store holds at least 5 time steps (one window and its label)", (long long)st->n_frames);
+    BC_CHECK_ARG(st->src_h >= BC_H && st->src_w >= BC_W, "bc_stage_gather: source frames %dx%d are smaller than %dx%d", st->src_h, st->src_w, BC_H, BC_W);
+    BC_CHECK_ARG(table || (st->src_h == BC_H && st->src_w == BC_W), "bc_stage_gather: %dx%d sources need a crop table", st->src_h, st->src_w);
+    BC_CHECK_ARG(out_dtype == BC_F32 || out_dtype == BC_BF16_TP, "bc_stage_gather: the output is BC_F32 or BC_BF16_TP planes, got %d", out_dtype);
+    BC_CHECK_ARG((uintptr_t)out % 16 == 0 && (uintptr_t)table % 16 == 0, "bc_stage_gather: out and table must be 16 B aligned");
+    BC_CHECK_ARG((uintptr_t)index % 8 == 0 && (uintptr_t)st->labels % 8 == 0 && (uintptr_t)st->commands % 8 == 0
+                 && (uintptr_t)st->targets % 4 == 0 && (uintptr_t)y % 8 == 0 && (uintptr_t)command % 8 == 0 && (uintptr_t)target % 4 == 0,
+                 "bc_stage_gather: index, labels, commands, y, command must be 8 B and targets, target 4 B aligned");
+    BC_CHECK_ARG(table || (uintptr_t)st->frames % 4 == 0, "bc_stage_gather: frames must be 4 B aligned");
+    BC_CHECK_ARG(!(st->targets && target) || st->n_out >= 1, "bc_stage_gather: n_out=%d must be at least 1 with targets", st->n_out);
+    const bool tp = out_dtype == BC_BF16_TP;
+    const int64_t units = (int64_t)batch * 4 * st->cams * (tp ? 3 * TP_NQ * TP_NU : BC_H * BC_W / 4);
+    BC_CHECK_ARG(units < (int64_t)0x7fffffff - 0x1000000, "bc_stage_gather: batch %d x %d cameras in one call (32-bit unit index)", batch, st->cams);
+    const int64_t cap = (int64_t)bc::num_sms() * 16;
+    const int blocks = (int)((units + 255) / 256 < cap ? (units + 255) / 256 : cap);
+    const AugRow* t = (const AugRow*)table;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tp && table)
+        bc::launch_pdl(stage_gather_kernel<true, true>, dim3(blocks), dim3(256), 0, s, *st, index, batch, t, out, y, command, target, err_flag, (uint32_t)units);
+    else if (tp)
+        bc::launch_pdl(stage_gather_kernel<true, false>, dim3(blocks), dim3(256), 0, s, *st, index, batch, t, out, y, command, target, err_flag, (uint32_t)units);
+    else if (table)
+        bc::launch_pdl(stage_gather_kernel<false, true>, dim3(blocks), dim3(256), 0, s, *st, index, batch, t, out, y, command, target, err_flag, (uint32_t)units);
+    else
+        bc::launch_pdl(stage_gather_kernel<false, false>, dim3(blocks), dim3(256), 0, s, *st, index, batch, t, out, y, command, target, err_flag, (uint32_t)units);
+    BC_CUDA_LAUNCH_CHECK("stage_gather_kernel");
     return BC_OK;
 }

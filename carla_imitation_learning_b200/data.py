@@ -11,13 +11,13 @@ zero-copy strided view -- 5.4x fewer PCIe bytes than f32 samples, 4x fewer conve
 """
 from __future__ import annotations
 
-from typing import Iterator, Optional, Tuple
+from typing import Callable, Iterator, Optional, Tuple
 
 import numpy as np
 import torch
 
 from . import _lib
-from .engine import StagedBatch, sliding_window, stage_frames, stage_gray
+from .engine import StagedBatch, _check_augment_table, _ptr, sliding_window, stage_frames, stage_gather, stage_gray
 
 
 def synthetic_sequence(seed: int, n_frames: int, h: int = 256, w: int = 256, n_actions: int = 9,
@@ -201,13 +201,203 @@ class SequentialFrames:
                 return
 
 
+def valid_starts(episode_lengths, frame_skip: int = 4) -> np.ndarray:
+    """EXTENSION: the sample indices of a store of episodes laid end to end (episode e holds time steps [o_e, o_e + L_e)) whose
+    window [i, i + frame_skip) and label frame i + frame_skip lie inside one episode: o_e .. o_e + L_e - frame_skip - 1 for
+    every episode, in order. This is what a ConcatDataset of per-episode SequentialTorchDatasets exposes
+    (imitation_dataset.py:90-136: L - frame_skip samples per episode); an episode of frame_skip frames or fewer has none."""
+    lengths = np.asarray(episode_lengths, dtype=np.int64).reshape(-1)
+    if (lengths < 0).any():
+        raise ValueError("episode lengths are non-negative")
+    offsets = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
+    parts = [o + np.arange(max(int(n) - frame_skip, 0), dtype=np.int64) for o, n in zip(offsets, lengths)]
+    return np.concatenate(parts) if parts else np.zeros(0, np.int64)
+
+
+class FrameStore:
+    """EXTENSION: a dataset's frames and side data in device memory, the source of shuffled minibatches (engine.stage_gather,
+    ShuffledFrames, TrainStep.step_gather). A B200 holds 200 K CARLA frames of 256 x 256 u8 RGB (39 GB).
+
+    frames_u8: (n_frames*cams, Hs, Ws, 3) u8, row t*cams + k = camera k at time t, Hs, Ws >= 256 (larger frames are cropped
+    by an augmentation table); labels (n_frames,) int64 class ids, commands (n_frames,) int64 branch ids, targets
+    (n_frames, n_out) f32 regression targets, each optional. numpy arrays or host tensors are uploaded once; CUDA tensors on
+    `device` are wrapped without a copy (they must then stay alive and unchanged while the store is in use). Several
+    episodes are laid end to end; valid_starts() names the samples that do not straddle two of them."""
+
+    def __init__(self, frames_u8, labels=None, commands=None, targets=None, cams: int = 1, device: Optional[torch.device] = None):
+        if cams not in (1, 3):
+            raise ValueError("cams is 1 (obs_size 4) or 3 (obs_size 12)")
+        if device is None:
+            device = frames_u8.device if isinstance(frames_u8, torch.Tensor) and frames_u8.is_cuda else \
+                torch.device("cuda", torch.cuda.current_device())
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("FrameStore lives in device memory; there is no CPU path")
+        fr = self._upload(frames_u8, torch.uint8, "frames")
+        if fr.dim() != 4 or fr.shape[-1] != 3 or fr.shape[1] < 256 or fr.shape[2] < 256 or fr.shape[0] % cams:
+            raise ValueError("frames must be (n_frames*cams, Hs, Ws, 3) uint8 with Hs, Ws >= 256")
+        self.frames, self.cams = fr, int(cams)
+        self.n_frames = fr.shape[0] // cams
+        if self.n_frames < 5:
+            raise ValueError("a store holds at least 5 time steps (one 4-frame window and the label after it)")
+        self.src_hw = (int(fr.shape[1]), int(fr.shape[2]))
+        self.labels = None if labels is None else self._upload(labels, torch.int64, "labels")
+        self.commands = None if commands is None else self._upload(commands, torch.int64, "commands")
+        self.targets = None if targets is None else self._upload(targets, torch.float32, "targets")
+        for name, t in (("labels", self.labels), ("commands", self.commands)):
+            if t is not None and tuple(t.shape) != (self.n_frames,):
+                raise ValueError(f"{name} are ({self.n_frames},): one per time step")
+        if self.targets is not None and (self.targets.dim() != 2 or self.targets.shape[0] != self.n_frames):
+            raise ValueError(f"targets are ({self.n_frames}, n_out): one row per time step")
+        self.n_out = 0 if self.targets is None else int(self.targets.shape[1])
+        self.n_samples = self.n_frames - 4
+        self.err_flag = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self.struct = _lib.BcFrameStore(self.frames.data_ptr(), self.n_frames, self.cams, self.src_hw[0], self.src_hw[1],
+                                        _ptr(self.labels), _ptr(self.commands), _ptr(self.targets), self.n_out)
+
+    def _upload(self, a, dtype: torch.dtype, what: str) -> torch.Tensor:
+        t = torch.from_numpy(np.ascontiguousarray(a)) if isinstance(a, np.ndarray) else a
+        if not isinstance(t, torch.Tensor):
+            raise ValueError(f"{what} must be a numpy array or a tensor")
+        if t.is_cuda:
+            if t.device != self.device or t.dtype != dtype or not t.is_contiguous():
+                raise ValueError(f"device {what} must be a contiguous {dtype} tensor on {self.device}")
+            return t
+        return t.to(dtype=dtype).contiguous().to(self.device)
+
+    def check(self) -> None:
+        """Raise if a staging launch met a sample index outside [0, n_frames - 5] (synchronises)."""
+        code = int(self.err_flag.item())
+        if code != 0:
+            self.err_flag.zero_()
+            raise RuntimeError(f"bc_stage_gather: a sample index outside [0, {self.n_frames - 5}] was staged (device flag {code})")
+
+
+class ShuffledFrames:
+    """EXTENSION: the shuffled counterpart of SequentialFrames -- minibatches of samples drawn at random from a FrameStore,
+    staged by ONE bc_stage_gather launch per batch (conditional imitation trains on such batches; a sequential batch is
+    ~13 s of one drive and may straddle two episodes).
+
+    Yields (x, y) like SequentialFrames, or (x, command, target) when the store has commands (the branched policy: target =
+    the store's targets when it has them, else its labels). x holds the windows materialised: layout 'plain' = a contiguous
+    (b, 4*cams, 256, 256) f32 tensor, 'tp' = a StagedBatch of Toeplitz-ready bf16 planes (precision='bf16').
+
+    Order: epoch e visits `starts` (default: every sample of the store; valid_starts() for episodes) in the order of a host
+    numpy PCG64 permutation seeded with seed + e, so it is reproducible and checkable on the CPU. Rank r of `world` takes
+    the disjoint shard permutation[r::world] (DistributedSampler's interleaving, without padding: shards differ by at most
+    one sample). The last batch may be short (no drop_last, as in the reference). Each __iter__ runs epoch `self.epoch`
+    and advances it (set it to resume at an epoch). table_fn(epoch, batch_idx, rows) -> (rows, 8) f32 rows of data.augment_table (rows =
+    b*cams), required for frames larger than 256x256: row b*cams + k applies to all four frames of camera k of sample b.
+
+    Index, side data, table and staging buffers rotate over two persistent device slots, as in SequentialFrames: a batch is
+    valid until the consumer has asked for two more, and its addresses repeat, so a CUDA-graph module step keeps replaying.
+    Everything is enqueued on the consumer's current stream; nothing synchronises the host."""
+
+    def __init__(self, store: FrameStore, batch_size: int, seed: int = 0, layout: str = "plain", starts=None,
+                 table_fn: Optional[Callable] = None, rank: int = 0, world: int = 1):
+        if layout not in ("plain", "tp"):
+            raise ValueError("layout is 'plain' (f32 planes) or 'tp' (Toeplitz-ready bf16 planes for precision='bf16')")
+        if not 0 <= rank < world:
+            raise ValueError(f"rank {rank} outside [0, {world})")
+        if int(batch_size) < 1:
+            raise ValueError("batch_size must be at least 1")
+        self.store, self.batch_size, self.seed, self.layout = store, int(batch_size), int(seed), layout
+        self.rank, self.world, self.table_fn, self.epoch = int(rank), int(world), table_fn, 0
+        self.starts = (np.arange(store.n_samples, dtype=np.int64) if starts is None
+                       else np.asarray(starts, dtype=np.int64).reshape(-1))
+        if self.starts.size == 0:
+            raise ValueError("no sample to draw")
+        if self.starts.min() < 0 or self.starts.max() > store.n_frames - 5:
+            raise ValueError(f"sample indices lie in [0, {store.n_frames - 5}]")
+        if store.src_hw != (256, 256) and table_fn is None:
+            raise ValueError(f"{store.src_hw[0]}x{store.src_hw[1]} frames need table_fn (crop rows, data.augment_table)")
+        dev, B, cams = store.device, self.batch_size, store.cams
+        self.branched = store.commands is not None
+        i64 = dict(dtype=torch.int64, device=dev)
+        self._idx = [torch.zeros(B, **i64) for _ in range(2)]
+        self._lab = [torch.zeros(B, **i64) for _ in range(2)] if store.labels is not None else None
+        self._cmd = [torch.zeros(B, **i64) for _ in range(2)] if self.branched else None
+        self._tgt = ([torch.zeros((B, store.n_out), dtype=torch.float32, device=dev) for _ in range(2)]
+                     if store.targets is not None else None)
+        self._tab = [torch.zeros((B * cams, 8), dtype=torch.float32, device=dev) for _ in range(2)] if table_fn else None
+        if layout == "tp":
+            self._x = [torch.empty((B * 4 * cams, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev) for _ in range(2)]
+        else:
+            self._x = [torch.empty((B, 4 * cams, 256, 256), dtype=torch.float32, device=dev) for _ in range(2)]
+        if self.branched and self._tgt is None and self._lab is None:
+            raise ValueError("a store with commands needs labels (CE) or targets (L1 / MSE)")
+        if not self.branched and self._lab is None:
+            raise ValueError("a store without commands needs labels")
+
+    def permutation(self, epoch: int) -> np.ndarray:
+        """Every start, in epoch `epoch`'s order (all ranks)."""
+        rng = np.random.Generator(np.random.PCG64(self.seed + int(epoch)))
+        return self.starts[rng.permutation(self.starts.size)]
+
+    def shard(self, epoch: int) -> np.ndarray:
+        """This rank's sample indices of epoch `epoch`, in the order they are staged."""
+        return self.permutation(epoch)[self.rank::self.world]
+
+    def __len__(self) -> int:
+        n = (self.starts.size - self.rank + self.world - 1) // self.world
+        return (n + self.batch_size - 1) // self.batch_size
+
+    def __iter__(self):
+        epoch = self.epoch
+        self.epoch += 1
+        order = self.shard(epoch)
+        store, B, cams = self.store, self.batch_size, self.store.cams
+        dev_order = torch.from_numpy(np.ascontiguousarray(order)).to(store.device)
+        for k in range((order.size + B - 1) // B):
+            slot, lo = k & 1, k * B
+            b = min(B, order.size - lo)
+            idx = self._idx[slot][:b]
+            idx.copy_(dev_order[lo:lo + b])
+            table = None
+            if self.table_fn is not None:
+                rows = self.table_fn(epoch, k, b * cams)
+                rows = torch.as_tensor(rows, dtype=torch.float32)
+                if tuple(rows.shape) != (b * cams, 8):
+                    raise ValueError(f"table_fn must return ({b * cams}, 8) float32 rows")
+                if rows.device.type == "cpu":
+                    _check_augment_table(rows, *store.src_hw)
+                table = self._tab[slot][:b * cams]
+                table.copy_(rows)
+            out = (StagedBatch(self._x[slot][:b * 4 * cams], None, 4 * cams, 4 * cams) if self.layout == "tp"
+                   else self._x[slot][:b])
+            lab = None if self._lab is None else self._lab[slot][:b]
+            cmd = None if self._cmd is None else self._cmd[slot][:b]
+            tgt = None if self._tgt is None else self._tgt[slot][:b]
+            x = stage_gather(store, idx, self.layout, out=out, table=table, y=lab, command=cmd, target=tgt)
+            if self.branched:
+                yield x, cmd, (tgt if tgt is not None else lab)
+            else:
+                yield x, lab
+
+
+def _datamodule_key(hparams, key: str, default):
+    """A configs/datamodule key: at the root of flat hparams, else in the composed config's `datamodule` group."""
+    if not hasattr(hparams, 'get'):
+        return default
+    if key in hparams:
+        return hparams[key]
+    group = hparams.get('datamodule')
+    return group.get(key, default) if hasattr(group, 'get') else default
+
+
 def sequential_train_val_test_iterator(hparams, frames_by_split=None):
     """{'train_dataloader','val_dataloader','test_dataloader'} like
     imitation_dataset.sequential_train_val_test_iterator (imitation_dataset.py:263-288).
     `frames_by_split` maps split -> (frames_u8, labels); without it a synthetic sequence is
-    generated (the reference ships no data, BASELINE.json asks for synthetic frames)."""
+    generated (the reference ships no data, BASELINE.json asks for synthetic frames).
+    With `shuffle: true` (configs/datamodule) the train split is a ShuffledFrames over a device FrameStore of its frames,
+    permuted per epoch from `shuffle_seed`; validation and test stay sequential."""
     bs = int(hparams['BATCH_SIZE'])
     fs = int(hparams.get('frame_skip', 4)) if hasattr(hparams, 'get') else int(hparams['frame_skip'])
+    bf16 = (hparams.get('precision', 'fp32') if hasattr(hparams, 'get') else 'fp32') == 'bf16'
+    shuffle, seed = bool(_datamodule_key(hparams, 'shuffle', False)), int(_datamodule_key(hparams, 'shuffle_seed', 0))
+    if shuffle and fs != 4:
+        raise ValueError("shuffled batches stage 4-frame windows: frame_skip must be 4")
     out = {}
     for i, split in enumerate(("train", "val", "test")):
         if frames_by_split is not None:
@@ -215,6 +405,8 @@ def sequential_train_val_test_iterator(hparams, frames_by_split=None):
         else:
             frames, labels = synthetic_sequence(i, (8 if split == "train" else 2) * bs + fs,
                                                 n_actions=int(hparams['n_actions']))
-        bf16 = (hparams.get('precision', 'fp32') if hasattr(hparams, 'get') else 'fp32') == 'bf16'
-        out[f"{split}_dataloader"] = SequentialFrames(frames, labels, bs, fs, layout="tp" if bf16 else "plain")
+        if shuffle and split == "train":
+            out["train_dataloader"] = ShuffledFrames(FrameStore(frames, labels), bs, seed, layout="tp" if bf16 else "plain")
+        else:
+            out[f"{split}_dataloader"] = SequentialFrames(frames, labels, bs, fs, layout="tp" if bf16 else "plain")
     return out

@@ -86,15 +86,26 @@ class StagedBatch:
 
     def __init__(self, tp: torch.Tensor, plain: Optional[torch.Tensor] = None, frame_skip: int = 4, step: int = 1):
         # step = planes a sample advances by: 1 = the reference's 4-frame window; 3 with frame_skip 12 = BASELINE configs[3],
-        # three cameras interleaved frame by frame (sample i = planes [3i, 3i+12), channel = 3*frame + camera)
+        # three cameras interleaved frame by frame (sample i = planes [3i, 3i+12), channel = 3*frame + camera);
+        # step == frame_skip = materialised windows that share no plane (stage_gather: shuffled samples)
         self.tp, self.plain, self.frame_skip, self.step = tp, plain, frame_skip, step
 
     @property
+    def materialised(self) -> bool:
+        return self.step == self.frame_skip
+
+    @property
     def x(self) -> Optional[torch.Tensor]:
-        return None if self.plain is None else sliding_window(self.plain, self.frame_skip, self.step)
+        if self.plain is None:
+            return None
+        if self.materialised:
+            return self.plain.view(-1, self.frame_skip, H, W)
+        return sliding_window(self.plain, self.frame_skip, self.step)
 
     @property
     def shape(self):
+        if self.materialised:
+            return (self.tp.shape[0] // self.step, self.frame_skip, H, W)
         return ((self.tp.shape[0] - self.frame_skip) // self.step, self.frame_skip, H, W)
 
     @property
@@ -182,6 +193,71 @@ def stage_augmented(frames_u8: torch.Tensor, table: torch.Tensor, layout: str = 
     if n:
         _lib.check(_lib.lib().bc_stage_augment(frames_u8.data_ptr(), n, hs, ws, table.data_ptr(), out.data_ptr(), code, _stream_ptr()), "bc_stage_augment")
     return res
+
+
+def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
+    return None if t is None else t.data_ptr()
+
+
+def stage_gather(store, index: torch.Tensor, layout: str = "tp", out=None, table: Optional[torch.Tensor] = None,
+                 y: Optional[torch.Tensor] = None, command: Optional[torch.Tensor] = None,
+                 target: Optional[torch.Tensor] = None, err_flag: Optional[torch.Tensor] = None):
+    """EXTENSION: B shuffled samples from a device-resident data.FrameStore in ONE staging launch (bc_stage_gather).
+    index (B,) int64 on the store's device: index[b] = i is the reference's sample i (frames i .. i+3, side data of frame
+    i+4). Returns the windows materialised, channel cams*j + k = camera k of frame i+j: layout 'tp' -> StagedBatch of B*4*cams
+    Toeplitz-ready bf16 planes (precision='bf16'), 'plain' -> a contiguous (B, 4*cams, 256, 256) f32 tensor. `out` = a
+    persistent destination of that form. table = (B*cams, 8) f32 rows (data.augment_table / center_crop_table layout), row
+    b*cams + k for all four frames of camera k of sample b; required for stores of frames larger than 256x256. y, command
+    (B,) int64 and target (B, n_out) f32 are filled from the store's labels / commands / targets in the same launch when
+    given. An index outside [0, n_frames - 5] zeroes that sample and sets err_flag (default: store.err_flag) to 5.
+    A host table is checked like stage_augmented's; device tensors are not read back."""
+    dev = store.device
+    if not isinstance(index, torch.Tensor) or index.device != dev or index.dtype != torch.int64 or index.dim() != 1 \
+            or not index.is_contiguous():
+        raise ValueError(f"index must be a contiguous (B,) int64 tensor on {dev}")
+    B, cams = index.shape[0], store.cams
+    if B < 1:
+        raise ValueError("index holds no sample")
+    hs, ws = store.src_hw
+    if table is not None:
+        if tuple(table.shape) != (B * cams, 8):
+            raise ValueError(f"the augmentation table is ({B * cams}, 8) float32: one row per sample and camera")
+        if table.device.type == "cpu":
+            table = table.to(dtype=torch.float32)
+            _check_augment_table(table, hs, ws)
+            table = table.to(dev)
+        if table.device != dev or table.dtype != torch.float32 or not table.is_contiguous():
+            raise ValueError(f"table must be a contiguous float32 tensor on {dev}")
+    elif (hs, ws) != (H, W):
+        raise ValueError(f"{hs}x{ws} frames need a crop table (data.augment_table / center_crop_table rows)")
+    n_planes = B * 4 * cams
+    if layout == "tp":
+        if out is None:
+            out = StagedBatch(torch.empty((n_planes, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev), None, 4 * cams, 4 * cams)
+        elif (not isinstance(out, StagedBatch) or tuple(out.tp.shape) != (n_planes, _lib.TP_PLANE_ELEMS) or not out.materialised
+              or out.frame_skip != 4 * cams or out.tp.dtype != torch.bfloat16 or out.tp.device != dev or not out.tp.is_contiguous()):
+            raise ValueError(f"out for layout 'tp' is a materialised StagedBatch of {n_planes} planes on {dev}")
+        code, dst = _lib.BC_BF16_TP, out.tp
+    elif layout == "plain":
+        if out is None:
+            out = torch.empty((B, 4 * cams, H, W), dtype=torch.float32, device=dev)
+        elif (not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or tuple(out.shape) != (B, 4 * cams, H, W)
+              or not out.is_contiguous() or out.device != dev):
+            raise ValueError(f"out for layout 'plain' is a contiguous ({B}, {4 * cams}, {H}, {W}) float32 tensor on {dev}")
+        code, dst = _lib.BC_F32, out
+    else:
+        raise ValueError("layout is 'plain' or 'tp'")
+    for name, t, dt, shape in (("y", y, torch.int64, (B,)), ("command", command, torch.int64, (B,)),
+                               ("target", target, torch.float32, (B, store.n_out))):
+        if t is not None and (not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != dt
+                              or tuple(t.shape) != shape or not t.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous {shape} {dt} tensor on {dev}")
+    flag = store.err_flag if err_flag is None else err_flag
+    with on_device(dev):
+        _lib.check(_lib.lib().bc_stage_gather(C.byref(store.struct), index.data_ptr(), B, _ptr(table), dst.data_ptr(), code,
+                                              _ptr(y), _ptr(command), _ptr(target), flag.data_ptr(), _stream_ptr()),
+                   "bc_stage_gather")
+    return out
 
 
 @dataclass
@@ -298,9 +374,9 @@ class BCEngine:
 
     def check_input(self, x):
         if isinstance(x, StagedBatch):
-            if not (self.conv_mode & 1) or (x.frame_skip, x.step) != (self.obs_size, self.obs_size // 4):
+            if not (self.conv_mode & 1) or x.frame_skip != self.obs_size or x.step not in (self.obs_size // 4, self.obs_size):
                 raise ValueError("a StagedBatch feeds the bf16 tensor-core mode (precision='bf16'): frame_skip 4 for obs_size 4, "
-                                 "stage_frames(frame_skip=12, step=3) for obs_size 12")
+                                 "stage_frames(frame_skip=12, step=3) for obs_size 12, or stage_gather's materialised windows")
             if x.device != self.device:
                 raise RuntimeError(f"x is on {x.device}, parameters on {self.device}")
             return x
@@ -470,7 +546,8 @@ class BCEngine:
 
     _ERRORS = {1: "a tcgen05 pipeline wait timed out inside a kernel (mbarrier protocol error)",
                3: "a label outside [0, n_actions) reached the CrossEntropy kernel (nn.CrossEntropyLoss raises on it too)",
-               4: "a command outside [0, n_branches) reached the branched heads (its output and gradient rows are zero)"}
+               4: "a command outside [0, n_branches) reached the branched heads (its output and gradient rows are zero)",
+               5: "a sample index outside [0, n_frames - 5] reached bc_stage_gather (its planes and side data are zero)"}
 
     def check_device_errors(self) -> None:
         """Host-side check of the device error flag (synchronises; call outside the hot loop, e.g. at epoch end)."""

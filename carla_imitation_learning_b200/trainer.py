@@ -28,17 +28,75 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .engine import (BCEngine, StagedBatch, StepBuffers, _stream_ptr, on_device, stage_augmented, stage_frames, stage_gray,
-                     sliding_window)
+from .engine import (BCEngine, StagedBatch, StepBuffers, _stream_ptr, on_device, stage_augmented, stage_frames, stage_gather,
+                     stage_gray, sliding_window)
 from .optim import FusedAdam
 
 
-class TrainStep:
+class _GatherInput:
+    """The shuffled input of a training step (step_gather): a lazily allocated buffer of B materialised windows (4*cams planes
+    per sample, written by bc_stage_gather from a data.FrameStore) and the switch of the step's buffers between it and the
+    sequential staging buffer that step() fills. The step's activation and gradient buffers are shared by both inputs."""
+
+    _gx = None
+    _seq_input = None
+
+    def _gather_x(self):
+        if self._gx is None:
+            cams, B, dev = self.eng.obs_size // 4, self.batch, self.eng.device
+            if self.bf16:
+                self._gx = StagedBatch(torch.empty((B * 4 * cams, _lib.TP_PLANE_ELEMS), dtype=torch.bfloat16, device=dev),
+                                       None, 4 * cams, 4 * cams)
+            else:
+                self._gx = torch.empty((B, 4 * cams, 256, 256), dtype=torch.float32, device=dev)
+        return self._gx
+
+    def _point(self, gathered: bool) -> None:
+        b = self.bufs
+        if self._seq_input is None:
+            self._seq_input = (b.x, b.x_tp, b.x_tp_strides)
+        if not gathered:
+            b.x, b.x_tp, b.x_tp_strides = self._seq_input
+        elif self.bf16:
+            x = self._gather_x()
+            b.x, b.x_tp, b.x_tp_strides = None, x.tp, (x.step * _lib.TP_PLANE_ELEMS, _lib.TP_PLANE_ELEMS)
+        else:
+            b.x = self._gather_x()
+
+    @staticmethod
+    def gather_key(store, index, table=None) -> tuple:
+        """The graph-cache key of step_gather: every field of the store's bc_frame_store (a captured graph holds the struct
+        by value -- frames, size and the labels / commands / targets pointers), the index buffer and the table buffer. Two
+        stores equal in all of these keep their data at the same addresses, so one may replay the other's graph."""
+        st = store.struct
+        return ("gather", *(getattr(st, f) for f, _ in st._fields_), index.data_ptr(),
+                None if table is None else table.data_ptr())
+
+    def _check_gather(self, store, index, src_hw) -> None:
+        dev, B = self.eng.device, self.batch
+        if getattr(store, "struct", None) is None or store.device != dev:
+            raise ValueError(f"store must be a data.FrameStore on {dev}")
+        if store.cams != self.eng.obs_size // 4:
+            raise ValueError(f"obs_size {self.eng.obs_size} takes a store of {self.eng.obs_size // 4} camera(s), got {store.cams}")
+        if store.src_hw != (src_hw or (256, 256)):
+            raise ValueError(f"this step stages {src_hw or (256, 256)} frames, the store holds {store.src_hw}")
+        if (not isinstance(index, torch.Tensor) or index.device != dev or index.dtype != torch.int64
+                or tuple(index.shape) != (B,) or not index.is_contiguous()):
+            raise ValueError(f"index must be a contiguous ({B},) int64 tensor on {dev}")
+
+
+class TrainStep(_GatherInput):
     """stage -> forward -> backward -> [exchange] -> Adam on one engine, captured per input slot.
 
     `step(frames_u8, labels)`: frames (B+frame_skip, 256, 256, 3) u8 and labels (B,) int64 already on the device. The
     first call for a given (frames, labels) buffer pair runs eagerly, the second captures a CUDA graph, later calls
-    replay it -- so a caller that rotates over a few device slots pays one graph launch per step."""
+    replay it -- so a caller that rotates over a few device slots pays one graph launch per step.
+
+    `step_gather(store, index)`: the same step on B shuffled samples of a data.FrameStore (256x256 frames, cams =
+    obs_size / 4, labels), index (B,) int64 on the device = the reference's sample ids. One bc_stage_gather launch stages
+    the windows and their labels into a persistent buffer, then the same enqueue runs. One CUDA graph per (store, index
+    buffer, keyed by gather_key): the graph reads the index buffer's contents on every replay, so a caller may
+    rewrite it in place."""
 
     def __init__(self, net, optimizer: FusedAdam, batch: int, *, group=None, exchange: Optional[str] = None,
                  overlap: Optional[bool] = None, graph: bool = True, dp_overlap: bool = False):
@@ -80,11 +138,7 @@ class TrainStep:
     def _enqueue(self, frames_u8: torch.Tensor, labels: torch.Tensor) -> None:
         self._stage(frames_u8)
         self.bufs.y = labels
-        if self.dp is not None:
-            self.dp(self.bufs)
-        else:
-            self.eng.enqueue_train(self.bufs)
-            self.opt.step_flat(self.eng.grads)
+        self._train()
 
     # ------------------------------------------------------------------ step
     def step(self, frames_u8: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
@@ -92,6 +146,7 @@ class TrainStep:
         if frames_u8.shape[0] != self.batch + 4 or labels.shape[0] != self.batch:
             raise ValueError(f"TrainStep was built for {self.batch} samples ({self.batch + 4} frames)")
         self.eng.ensure_packed()
+        self._point(False)
         key = (frames_u8.data_ptr(), labels.data_ptr())
         g = self._graphs.get(key) if self.graph else None
         if g is not None:
@@ -104,18 +159,54 @@ class TrainStep:
             self._enqueue(frames_u8, labels)
         return self.bufs.loss
 
-    def _capture(self, frames_u8, labels):
+    def _capture(self, frames_u8, labels, pre=None):
         from .parallel import DataParallelStep
         self.opt.prepare()
-        if isinstance(self.dp, DataParallelStep):        # NCCL stays outside the graphs: three segments
+        if pre is None:
             def pre():
                 self._stage(frames_u8)
                 self.bufs.y = labels
+        if isinstance(self.dp, DataParallelStep):        # NCCL stays outside the graphs: three segments
             return self.dp.capture(self.bufs, pre)
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
-            self._enqueue(frames_u8, labels)
+            pre()
+            self._train()
         return g
+
+    def _train(self) -> None:
+        if self.dp is not None:
+            self.dp(self.bufs)
+        else:
+            self.eng.enqueue_train(self.bufs)
+            self.opt.step_flat(self.eng.grads)
+
+    def step_gather(self, store, index: torch.Tensor) -> torch.Tensor:
+        """Enqueue one optimisation step on the shuffled samples `index` of `store` (a data.FrameStore); returns the
+        (device) loss cell. An index outside [0, n_frames - 5] trains on a zero window with label 0 and raises at check()."""
+        self._check_gather(store, index, None)
+        if store.labels is None:
+            raise ValueError("the store has no labels")
+        self.eng.ensure_packed()
+        self._point(True)
+        x = self._gather_x()
+        if getattr(self, "_gy", None) is None:
+            self._gy = torch.zeros(self.batch, dtype=torch.int64, device=self.eng.device)
+
+        def pre():
+            stage_gather(store, index, "tp" if self.bf16 else "plain", out=x, y=self._gy, err_flag=self.eng.err_flag)
+            self.bufs.y = self._gy
+        key = self.gather_key(store, index)
+        g = self._graphs.get(key) if self.graph else None
+        if g is None and self.graph and key in self._seen:
+            g = self._graphs[key] = self._capture(None, None, pre)
+        if g is not None:
+            self._replay(g)
+        else:
+            self._seen.add(key)
+            pre()
+            self._train()
+        return self.bufs.loss
 
     def _replay(self, g) -> None:
         from .parallel import DataParallelStep
@@ -200,7 +291,7 @@ class _BranchedInput:
             stage_gray(frames_u8, out=self.gray)
 
 
-class BranchedTrainStep(_BranchedInput):
+class BranchedTrainStep(_BranchedInput, _GatherInput):
     """stage [+ augment] -> conv1..4 -> branched heads + loss + backward -> trunk backward -> Adam on both arenas, for a
     ConvNet1Branched and its MultiArenaAdam at a static batch, captured per input slot like TrainStep.
 
@@ -209,7 +300,13 @@ class BranchedTrainStep(_BranchedInput):
     kernel), None when src_hw is None (plain staging of 256x256 frames); command (B,) int64 branch ids; target (B,) int64
     class ids for branch_loss 'ce', (B, n_out) f32 for 'l1' / 'mse'. The first call for a given buffer tuple runs
     eagerly, the second captures a CUDA graph, later calls replay it. Returns the device loss cell, rewritten by the next
-    step. Nothing in step() synchronises the host; check() does."""
+    step. Nothing in step() synchronises the host; check() does.
+
+    `step_gather(store, index, table=None)`: the same step on B shuffled samples of a data.FrameStore (one camera, frames
+    of src_hw or 256x256, commands, and labels for 'ce' or targets for 'l1' / 'mse'); index (B,) int64 on the device;
+    table (B, 8) f32 rows on the device when built with src_hw (row b for all four frames of sample b), else None. One
+    bc_stage_gather launch stages the windows, commands and targets; one CUDA graph per (store, index buffer, table
+    buffer), which reads their contents on every replay."""
 
     def __init__(self, net, optimizer, batch: int, *, src_hw=None, graph: bool = True, group=None):
         if dist.is_initialized() and dist.get_world_size(group) > 1:
@@ -245,6 +342,9 @@ class BranchedTrainStep(_BranchedInput):
 
     def _enqueue(self, frames_u8, table, command, target) -> None:
         self._stage(frames_u8, table)
+        self._train(command, target)
+
+    def _train(self, command, target) -> None:
         self.eng.enqueue_trunk_forward(self.bufs)
         self.net._head(self.bufs, self.hb, command, target, 3)      # outputs, loss, dout, branch gradients, ghead
         self.eng.enqueue_trunk_backward(self.bufs)
@@ -257,21 +357,58 @@ class BranchedTrainStep(_BranchedInput):
         """Enqueue one optimisation step; returns the (device) loss cell, rewritten by the next step."""
         self._check_inputs(frames_u8, table, command, target)
         self.eng.ensure_packed()
+        self._point(False)
         key = (frames_u8.data_ptr(), None if table is None else table.data_ptr(), command.data_ptr(), target.data_ptr())
+        return self._run(key, lambda: self._enqueue(frames_u8, table, command, target))
+
+    def _run(self, key, enqueue) -> torch.Tensor:
         g = self._graphs.get(key) if self.graph else None
         if g is None and self.graph and key in self._seen:
             self.opt.prepare()
             g = self._graphs[key] = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self._enqueue(frames_u8, table, command, target)
+                enqueue()
         if g is not None:
             self.opt.prepare()            # an LR milestone reaches the device scalars the captured Adam kernels read
             g.replay()
         else:
             self._seen.add(key)
             self.opt.prepare()
-            self._enqueue(frames_u8, table, command, target)
+            enqueue()
         return self.hb["loss"]
+
+    def step_gather(self, store, index: torch.Tensor, table: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Enqueue one optimisation step on the shuffled samples `index` of `store`; returns the (device) loss cell. An index
+        outside [0, n_frames - 5] trains on a zero window with command 0 and a zero target and raises at check()."""
+        self._check_gather(store, index, self.src_hw)
+        B, dev, ce = self.batch, self.eng.device, self.net.branch_loss == "ce"
+        if self.src_hw is None:
+            if table is not None:
+                raise ValueError("this step was built without augmentation (src_hw=None): table must be None")
+        elif (not isinstance(table, torch.Tensor) or table.device != dev or table.dtype != torch.float32
+              or tuple(table.shape) != (B, 8) or not table.is_contiguous()):
+            raise ValueError(f"table must be a contiguous ({B}, 8) float32 tensor on {dev} (data.augment_table rows)")
+        if store.commands is None:
+            raise ValueError("the store has no commands")
+        if ce and store.labels is None:
+            raise ValueError("branch_loss 'ce' needs a store with labels")
+        if not ce and (store.targets is None or store.n_out != self.net.n_actions):
+            raise ValueError(f"branch_loss '{self.net.branch_loss}' needs a store with ({self.net.n_actions},) target rows")
+        self.eng.ensure_packed()
+        self._point(True)
+        x = self._gather_x()
+        if getattr(self, "_gside", None) is None:
+            self._gside = (torch.zeros(B, dtype=torch.int64, device=dev),
+                           torch.zeros(B, dtype=torch.int64, device=dev) if ce else
+                           torch.zeros((B, self.net.n_actions), dtype=torch.float32, device=dev))
+        command, target = self._gside
+
+        def enqueue():
+            stage_gather(store, index, "tp" if self.bf16 else "plain", out=x, table=table, command=command,
+                         y=target if ce else None, target=None if ce else target, err_flag=self.eng.err_flag)
+            self._train(command, target)
+        key = self.gather_key(store, index, table)
+        return self._run(key, enqueue)
 
     @property
     def out(self) -> torch.Tensor:

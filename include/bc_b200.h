@@ -130,6 +130,37 @@ int bc_stage_augment(const uint8_t* rgb, int64_t n_frames, int src_h, int src_w,
 int bc_stage_history(const uint8_t* rgb, int n_agents, int cams, int src_h, int src_w, const float* table,
                      const uint8_t* reset, int reset_all, void* ring, int slot, int out_dtype, void* stream);
 
+/* EXTENSION: shuffled minibatches from a frame store that lives in device memory (a dataset uploaded once; a B200 holds 200 K
+ * CARLA frames of 256x256 u8 RGB in 39 GB). frames: (n_frames*cams, src_h, src_w, 3) u8, row t*cams + k = camera k at time t;
+ * labels, commands: (n_frames,) int64 or NULL; targets: (n_frames, n_out) f32 or NULL. Offsets into the store are 64-bit. */
+typedef struct {
+    const uint8_t* frames;
+    int64_t n_frames;        /* time steps in the store */
+    int32_t cams, src_h, src_w;
+    const int64_t* labels;   /* (n_frames,) or NULL */
+    const int64_t* commands; /* (n_frames,) or NULL (branched policy) */
+    const float* targets;    /* (n_frames, n_out) or NULL (L1 / MSE)   */
+    int32_t n_out;
+} bc_frame_store;
+
+/* Stage `batch` samples drawn anywhere in the store in ONE launch. index (batch,) int64: index[b] = i names the reference's
+ * sample i (SequentialTorchDataset.__getitem__, src/dataset/imitation_dataset.py:117-131): frames i .. i+3 and the label,
+ * command and target of frame i+4. Output plane b*4*cams + cams*j + k is camera k of frame i+j -- the channel order of the
+ * sliding window, materialised: conv1 reads it with (x_stride_n, x_stride_c) = (4*cams, 1) planes. BC_F32: a contiguous
+ * (batch, 4*cams, 256, 256) tensor; BC_BF16_TP: batch*4*cams Toeplitz-ready planes. table NULL (256x256 sources only): every
+ * plane is bitwise what bc_stage_gray(BC_F32) / bc_stage_gray_tp writes for its source frame; table ((batch*cams, 8) f32 rows,
+ * data.augment_table layout): row b*cams + k applies to all four frames of camera k of sample b (crop and jitter consistent
+ * in time within a window), bitwise what bc_stage_augment writes for that frame and row. y (batch,) int64, command (batch,)
+ * int64 and target (batch, n_out) f32 are written when both their pointer and the store's array are non-NULL. An index outside
+ * [0, n_frames - 5] sets *err_flag = 5 unless it already holds a nonzero code, and gives that sample zero planes, label 0, command 0 and a zero target row; nothing
+ * outside the store is read. Arguments are checked before any CUDA call: non-NULL store, frames, index, out and err_flag,
+ * batch >= 1, cams in {1, 3}, n_frames >= 5, src >= 256 and a table for sources that are not 256x256, out and table 16 B
+ * aligned, at most 2^31 - 2^24 units (the unit index is 32-bit). Launched with programmatic stream serialisation: index and
+ * table are read before the kernel waits for its predecessor, every store comes after (the previous step's conv1 forward and
+ * weight gradient read the planes this launch overwrites). */
+int bc_stage_gather(const bc_frame_store* s, const int64_t* index, int batch, const float* table, void* out, int out_dtype,
+                    int64_t* y, int64_t* command, float* target, int32_t* err_flag, void* stream);
+
 /* plain planes (f32 or bf16; 256x256, rows contiguous, `plane_stride` elements apart) -> BC_BF16_TP planes:
  * how a reference-style (B,4,256,256) batch enters the tcgen05 conv1 (bf16 mode) */
 int bc_planes_to_tp(const void* planes, int in_dtype, int64_t n_planes, int64_t plane_stride, void* out_tp, void* stream);
@@ -177,7 +208,8 @@ int bc_loss_reduce(const bc_ctx* c, void* stream);                 /* head CTAs'
  * and never from a kernel of its own that calls griddepcontrol.launch_dependents before its last write. The same holds for
  * the command vector of the branched serving tail (bc_policy_tail_branched), which reads command[b] before its wait: no
  * kernel of this library writes it. No kernel of this library writes the reset vector of bc_stage_history either: the caller
- * writes it with stream-ordered work, as it does the command vector. */
+ * writes it with stream-ordered work, as it does the command vector. The same holds for the index vector (and the table) of
+ * bc_stage_gather, and for the frame store itself: no kernel of this library writes them. */
 
 /* ---- a11: Adam.step (src/models/imitation.py:82-87; torch.optim.Adam defaults).
  * state = 8 DOUBLES {lr, beta1, beta2, eps, step, grad_scale, step_size(out), bc2_sqrt(out)} on the
