@@ -53,7 +53,7 @@ class BcBranched(C.Structure):
                 ("feat", C.c_void_p), ("command", C.c_void_p), ("labels", C.c_void_p), ("targets", C.c_void_p),
                 ("params", C.c_void_p), ("grads", C.c_void_p), ("out", C.c_void_p), ("dout", C.c_void_p),
                 ("gfeat", C.c_void_p), ("loss", C.c_void_p), ("partials", C.c_void_p), ("err_flag", C.c_void_p),
-                ("loss_scale", C.c_float)]
+                ("loss_scale", C.c_float), ("grads_epoch", C.c_void_p), ("grads_stride", C.c_int64)]
 
 
 class BcFrameStore(C.Structure):
@@ -92,6 +92,9 @@ EXPORTS = {
                                     C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "bc_adam_step_exchange": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(BcPeer),
                                         C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "bc_adam_step_exchange_arenas": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.POINTER(BcPeer), C.c_void_p,
+                                               C.c_int, C.c_int, C.c_void_p]),
     "bc_backward_overlap": (C.c_int, [C.POINTER(BcCtx), C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p), C.c_int]),
     "bc_argmax": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "bc_forward_act": (C.c_int, [C.POINTER(BcCtx), C.c_void_p, C.c_int, C.c_void_p]),

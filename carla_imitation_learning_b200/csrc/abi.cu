@@ -2,6 +2,7 @@
 #include "bc_common.cuh"
 #include "pack.cuh"
 #include <math.h>
+#include <type_traits>
 
 namespace bc {
 
@@ -213,12 +214,23 @@ struct ExchangeArgs {
     int* err;
     ctc::PackMap pm;
 };
+// Two arenas in one exchange (bc_adam_step_exchange_arenas): each half of the gradient buffer is [arena 0 | arena 1];
+// float4 i < split4 belongs to arena 0 (p, m, v, st above; the operand images follow it), the rest to arena 1.
+struct ExchangeArgs2 : ExchangeArgs {
+    float4* p2; float4* m2; float4* v2; double* st2;
+    int64_t split4;
+};
+template <int NSEG> using ExchangeArgsN = std::conditional_t<NSEG == 1, ExchangeArgs, ExchangeArgs2>;
 
-__global__ void __launch_bounds__(128) adam_exchange_kernel(const ExchangeArgs a) {
+template <int NSEG>
+__global__ void __launch_bounds__(128) adam_exchange_kernel(const ExchangeArgsN<NSEG> a) {
     __shared__ int s_last;
-    __shared__ double s_sc[3];
+    __shared__ double s_sc[3 * NSEG];
     bc::pdl_wait();                                         // no early release of the dependents: this kernel writes the parameters (see adam_tick_step_kernel)
-    if (threadIdx.x == 0) adam_scalars(a.st, s_sc);        // the tick is folded in (published by the last CTA of the publishing launch)
+    if (threadIdx.x == 0) {                                 // the tick is folded in (published by the last CTA of the publishing launch)
+        adam_scalars(a.st, s_sc);
+        if constexpr (NSEG == 2) adam_scalars(a.st2, s_sc + 3);
+    }
     const uint32_t epoch = a.sync[0] + 1;
     const int64_t par = (int64_t)(epoch & 1u) * a.arena4;
     uint32_t* my_sig = a.peer_signals[a.rank];
@@ -233,17 +245,25 @@ __global__ void __launch_bounds__(128) adam_exchange_kernel(const ExchangeArgs a
     if (!ok) return;                                        // parameters, moments, step count and epoch stay as they were
     // ---- B
     const AdamK k = adam_consts(a.st, s_sc[1], s_sc[2]);
+    AdamK k2 = k;
+    if constexpr (NSEG == 2) k2 = adam_consts(a.st2, s_sc[4], s_sc[5]);
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = a.lo4 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.hi4; i += stride) {
-        float4 pp = a.p[i], mm = a.m[i], vv = a.v[i];               // local state first: in flight under the NVLink round trips
+        float4 *p = a.p, *m = a.m, *v = a.v;
+        int64_t j = i;
+        bool first = true;
+        if constexpr (NSEG == 2) {
+            if (i >= a.split4) { p = a.p2; m = a.m2; v = a.v2; j = i - a.split4; first = false; }
+        }
+        float4 pp = p[j], mm = m[j], vv = v[j];                     // local state first: in flight under the NVLink round trips
         float4 gg = ld_relaxed_sys_f4(a.peer_grads[0] + par + i);
         for (int r = 1; r < a.world; ++r) {
             const float4 o = ld_relaxed_sys_f4(a.peer_grads[r] + par + i);
             gg.x = __fadd_rn(gg.x, o.x); gg.y = __fadd_rn(gg.y, o.y); gg.z = __fadd_rn(gg.z, o.z); gg.w = __fadd_rn(gg.w, o.w);
         }
-        adam4(pp, gg, mm, vv, k);
-        a.p[i] = pp; a.m[i] = mm; a.v[i] = vv;
-        ctc::pack_updated4(a.pm, 4 * i, &pp.x);
+        adam4(pp, gg, mm, vv, first ? k : k2);
+        p[j] = pp; m[j] = mm; v[j] = vv;
+        if (first) ctc::pack_updated4(a.pm, 4 * i, &pp.x);          // the operand images belong to arena 0 only
     }
     // ---- C
     if (!a.publish) return;
@@ -253,7 +273,10 @@ __global__ void __launch_bounds__(128) adam_exchange_kernel(const ExchangeArgs a
         s_last = atomicAdd(a.sync + 1, 1u) == gridDim.x - 1;
     }
     __syncthreads();
-    if (s_last && threadIdx.x == 0) { a.sync[1] = 0; a.sync[0] = epoch; a.st[4] = s_sc[0]; a.st[6] = s_sc[1]; a.st[7] = s_sc[2]; }
+    if (s_last && threadIdx.x == 0) {
+        if constexpr (NSEG == 2) { a.st2[4] = s_sc[3]; a.st2[6] = s_sc[4]; a.st2[7] = s_sc[5]; }
+        a.sync[1] = 0; a.sync[0] = epoch; a.st[4] = s_sc[0]; a.st[6] = s_sc[1]; a.st[7] = s_sc[2];
+    }
     // early returns above release the dependents implicitly when the grid completes
 }
 
@@ -388,7 +411,34 @@ int bc_adam_step_exchange(float* params, float* exp_avg, float* exp_avg_sq, doub
     int blocks = (int)((a.hi4 - a.lo4 + 127) / 128);           // one float4 per thread: a single NVLink round trip per thread
     const int cap = 2 * bc::num_sms();                         // every CTA spins on the flags: all of them must be resident
     if (blocks > cap) blocks = cap;
-    bc::launch_pdl(adam_exchange_kernel, dim3(blocks), dim3(128), 0, (cudaStream_t)stream, a);
+    bc::launch_pdl(adam_exchange_kernel<1>, dim3(blocks), dim3(128), 0, (cudaStream_t)stream, a);
+    BC_CUDA_LAUNCH_CHECK("adam_exchange_kernel");
+    return BC_OK;
+}
+
+int bc_adam_step_exchange_arenas(float* params, float* exp_avg, float* exp_avg_sq, double* state9,
+                                 float* params_b, float* exp_avg_b, float* exp_avg_sq_b, double* state9_b,
+                                 int64_t n, int64_t split, const bc_peer* peer, void* w_packed, int obs_size, int n_actions,
+                                 void* stream) {
+    BC_CHECK_ARG(params && exp_avg && exp_avg_sq && state9 && params_b && exp_avg_b && exp_avg_sq_b && state9_b && peer,
+                 "bc_adam_step_exchange_arenas: null pointer");
+    BC_CHECK_ARG(peer->peer_grads_dev && peer->peer_signals_dev && peer->sync_state && peer->err_flag, "bc_adam_step_exchange_arenas: null pointer in bc_peer");
+    BC_CHECK_ARG(n > 0 && n % 4 == 0, "bc_adam_step_exchange_arenas: n=%lld must be a positive multiple of 4", (long long)n);
+    BC_CHECK_ARG(0 < split && split < n && split % 4 == 0, "bc_adam_step_exchange_arenas: split %lld outside (0, %lld) or not a multiple of 4", (long long)split, (long long)n);
+    BC_CHECK_ARG(peer->world >= 1 && peer->world <= 64 && peer->rank >= 0 && peer->rank < peer->world, "bc_adam_step_exchange_arenas: rank %d of %d", peer->rank, peer->world);
+    BC_CHECK_ARG(((uintptr_t)params | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)params_b | (uintptr_t)exp_avg_b |
+                  (uintptr_t)exp_avg_sq_b) % 16 == 0, "bc_adam_step_exchange_arenas: 16 B alignment");
+    ExchangeArgs2 a{};
+    if (int rc = pack_map_for(&a.pm, w_packed, obs_size, n_actions, split, "bc_adam_step_exchange_arenas")) return rc;
+    a.p = (float4*)params; a.peer_grads = (const float4* const*)peer->peer_grads_dev; a.peer_signals = (uint32_t* const*)peer->peer_signals_dev;
+    a.m = (float4*)exp_avg; a.v = (float4*)exp_avg_sq; a.st = state9; a.sync = peer->sync_state;
+    a.p2 = (float4*)params_b; a.m2 = (float4*)exp_avg_b; a.v2 = (float4*)exp_avg_sq_b; a.st2 = state9_b; a.split4 = split / 4;
+    a.lo4 = 0; a.hi4 = n / 4; a.arena4 = n / 4;
+    a.rank = peer->rank; a.world = peer->world; a.bucket = 1; a.publish = 1; a.err = peer->err_flag;
+    int blocks = (int)((a.hi4 + 127) / 128);                   // one float4 per thread, as above
+    const int cap = 2 * bc::num_sms();                         // every CTA spins on the flags: all of them must be resident
+    if (blocks > cap) blocks = cap;
+    bc::launch_pdl(adam_exchange_kernel<2>, dim3(blocks), dim3(128), 0, (cudaStream_t)stream, a);
     BC_CUDA_LAUNCH_CHECK("adam_exchange_kernel");
     return BC_OK;
 }

@@ -263,10 +263,12 @@ __global__ void __launch_bounds__(NT) head_branched_kernel(const BrArgs a) {
     }
 }
 
-// grads[g][i] = sum over the branch's nb partial copies, in slot order; loss = sum of all loss partials
+// grads[g][i] = sum over the branch's nb partial copies, in slot order; loss = sum of all loss partials.
+// grads_epoch != NULL (data-parallel peer exchange): grads is double-buffered, the half ((*grads_epoch + 1) & 1) is written
 __global__ void __launch_bounds__(256) branched_reduce_kernel(const float* __restrict__ part, const float* __restrict__ loss_part,
                                                                float* __restrict__ grads, float* __restrict__ loss,
-                                                               int64_t len, int G, int nb, int with_grads, int with_loss) {
+                                                               int64_t len, int G, int nb, int with_grads, int with_loss,
+                                                               const uint32_t* __restrict__ grads_epoch, int64_t grads_stride) {
     bc::pdl_wait();
     bc::pdl_trigger();
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -275,7 +277,8 @@ __global__ void __launch_bounds__(256) branched_reduce_kernel(const float* __res
         const int64_t e = i - (int64_t)g * len;
         float s = 0.f;
         for (int k = 0; k < nb; ++k) s += part[((size_t)g * nb + k) * len + e];
-        grads[i] = s;
+        const int64_t par = grads_epoch ? (int64_t)((*grads_epoch + 1u) & 1u) * grads_stride : 0;
+        grads[par + i] = s;
     }
     if (with_loss && blockIdx.x == 0 && threadIdx.x < 32) {
         float v = 0.f;
@@ -328,7 +331,8 @@ static int head_branched_launch(const bc_branched* h, int mode, int64_t* actions
     if (mode & 3) {
         const int64_t n = a.L.len * a.G;
         bc::launch_pdl(branched_reduce_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
-                       (const float*)a.part, (const float*)a.loss_part, h->grads, h->loss, a.L.len, a.G, a.nb, (mode & 2) ? 1 : 0, (mode & 1) ? 1 : 0);
+                       (const float*)a.part, (const float*)a.loss_part, h->grads, h->loss, a.L.len, a.G, a.nb, (mode & 2) ? 1 : 0, (mode & 1) ? 1 : 0,
+                       h->grads_epoch, h->grads_stride);
         BC_CUDA_LAUNCH_CHECK("branched_reduce_kernel");
     }
     return BC_OK;

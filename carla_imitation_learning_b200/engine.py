@@ -459,8 +459,8 @@ class BCEngine:
         optimiser recognise .grad tensors that are views of one arena and consume it without a copy."""
         cands = [self.grads] + (self._slots or []) + ([self._last_flat] if getattr(self, "_last_flat", None) is not None else [])
         if self.peer is not None:
-            n = self.peer.n
-            cands = [self.peer.buf[:n], self.peer.buf[n:]] + cands[1:]
+            S = self.peer.stride
+            cands = [self.peer.buf[:S], self.peer.buf[S:]] + cands[1:]
         for t in cands:
             if t.data_ptr() == ptr and t.numel() >= self.arena.numel():
                 return t[:self.arena.numel()]

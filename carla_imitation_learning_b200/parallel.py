@@ -76,15 +76,19 @@ class GradExchange:
 
 class PeerGrads:
     """This rank's gradients in a symmetric allocation every rank maps (torch symmetric memory = cudaIpc / fabric handles;
-    plumbing): TWO arenas back to back -- step e writes and exchanges arena e & 1, so no "done reading" handshake is needed
-    (csrc/abi.cu) -- plus the per-rank signal pad and the private sync words of bc_adam_step_exchange."""
+    plumbing): TWO halves back to back -- step e writes and exchanges half e & 1, so no "done reading" handshake is needed
+    (csrc/abi.cu) -- plus the per-rank signal pad and the private sync words of bc_adam_step_exchange.
 
-    def __init__(self, engine, group: Optional[dist.ProcessGroup] = None):
+    A half is the engine's arena (n floats), followed by `extra` floats of a second arena when one exchange covers two
+    (the branched policy's branch arena, BranchedPeerExchange): stride = n + extra floats between the halves."""
+
+    def __init__(self, engine, group: Optional[dist.ProcessGroup] = None, extra: int = 0):
         import torch.distributed._symmetric_memory as symm
         group = group if group is not None else dist.group.WORLD
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.n = n = engine.arena.numel()
-        self.buf = symm.empty(2 * n, dtype=torch.float32, device=engine.device)
+        self.stride = S = n + int(extra)
+        self.buf = symm.empty(2 * S, dtype=torch.float32, device=engine.device)
         self.hdl = symm.rendezvous(self.buf, group.group_name)
         self.buf.zero_()
         self.hdl.get_signal_pad(self.rank).zero_()
@@ -94,15 +98,15 @@ class PeerGrads:
                                     self.err.data_ptr(), self.rank, self.world)
         self.host_epoch = 0                           # mirrors sync[0]: one per completed (publishing) exchange launch
         # backward now reduces its partial sums straight into peer-visible memory, into the half the device epoch selects
-        engine.grads, engine.grads_epoch, engine.grads_stride, engine.peer = self.buf, self.sync, n, self
+        engine.grads, engine.grads_epoch, engine.grads_stride, engine.peer = self.buf, self.sync, S, self
         self.buckets = grad_buckets(engine.obs_size, engine.n_actions)
         torch.cuda.synchronize(engine.device)
         dist.barrier(group)                           # every pad is zero before anybody signals
 
     def current(self) -> torch.Tensor:
-        """The arena the NEXT exchange reads (= the one the backward of the current step writes)."""
+        """The half the NEXT exchange reads (= the one the backward of the current step writes): stride floats."""
         half = (self.host_epoch + 1) & 1
-        return self.buf[half * self.n:(half + 1) * self.n]
+        return self.buf[half * self.stride:(half + 1) * self.stride]
 
     def check(self) -> None:
         if int(self.err.item()) != 0:
@@ -182,6 +186,51 @@ class ModuleExchange:
         if flat_grads.data_ptr() != cur.data_ptr():
             cur.copy_(flat_grads)
         self.opt.step_exchange(self.peer)
+        self.peer.host_epoch += 1
+
+
+class BranchedPeerExchange:
+    """The peer exchange of the command-conditioned branched policy (ConvNet1Branched + its MultiArenaAdam): each half of
+    the peer-visible gradient buffer is [trunk arena | branch arena]. The trunk backward (bc_ctx.grads_epoch) and the
+    branched heads' reduction (bc_branched.grads_epoch) write their gradients straight into the half the next exchange
+    reads; one bc_adam_step_exchange_arenas launch then sums all ranks' halves in rank order, folds the 1/world mean and
+    applies Adam to both arenas. Used by BranchedTrainStep (inside its CUDA graph) and, through MultiArenaAdam.step, by
+    the module path."""
+
+    def __init__(self, net, optimizer, group: Optional[dist.ProcessGroup] = None):
+        self.trunk_opt, self.branch_opt = optimizer.children_
+        self.peer = PeerGrads(net.engine(), group, extra=net._barena.numel())
+        for c in optimizer.children_:
+            c.set_grad_scale(1.0 / self.peer.world)
+        optimizer.prepare()
+        optimizer.exchange = self
+
+    def head_grads(self) -> dict:
+        """The bc_branched gradient fields of the heads' backward: the branch arena of half 0 + the epoch word."""
+        p = self.peer
+        return dict(grads=p.buf[p.n:], grads_epoch=p.sync, grads_stride=p.stride)
+
+    def exchange(self) -> None:
+        """Enqueue the two-arena exchange + Adam launch (after both arenas' gradients of this step are complete)."""
+        (pt, mt, vt, st, _), (pb, mb, vb, sb, _) = self.trunk_opt._bind(), self.branch_opt._bind()
+        if not torch.cuda.is_current_stream_capturing():
+            self.trunk_opt._sync_scalars(st)
+            self.branch_opt._sync_scalars(sb)
+        wp, obs, na = self.trunk_opt._packed()
+        with on_device(pt.device):
+            _lib.check(_lib.lib().bc_adam_step_exchange_arenas(
+                pt.data_ptr(), mt.data_ptr(), vt.data_ptr(), st.data_ptr(), pb.data_ptr(), mb.data_ptr(), vb.data_ptr(),
+                sb.data_ptr(), self.peer.stride, self.peer.n, self.peer.c_struct, wp, obs, na,
+                torch.cuda.current_stream(pt.device).cuda_stream), "bc_adam_step_exchange_arenas")
+
+    def step_from(self, trunk_grads: torch.Tensor, branch_grads: torch.Tensor) -> None:
+        """Module path (MultiArenaAdam.step): this rank's gradients of both arenas -> the current half (copied unless they
+        already sit there), then one exchange launch."""
+        cur, n = self.peer.current(), self.peer.n
+        for dst, g in ((cur[:n], trunk_grads), (cur[n:], branch_grads)):
+            if g.data_ptr() != dst.data_ptr():
+                dst.copy_(g)
+        self.exchange()
         self.peer.host_epoch += 1
 
 

@@ -6,8 +6,9 @@ Three layers:
 * TrainStep -- one optimisation step for a static batch shape, straight on the engine (no autograd): stage -> conv1..4 ->
   head + CE -> backward -> [peer exchange] -> Adam as ONE CUDA graph per input slot. This is what bench.py times as `value`
   and what Trainer.fit uses when the module is a ConvNet1-backed Imitation with `cuda_graph: true`.
-* BranchedTrainStep -- the same for the command-conditioned ConvNet1Branched (one GPU): stage [+ augment] -> conv1..4 ->
-  branched heads + CE / L1 / MSE -> trunk backward -> Adam on the trunk and the branch arena, one CUDA graph per input slot.
+* BranchedTrainStep -- the same for the command-conditioned ConvNet1Branched: stage [+ augment] -> conv1..4 -> branched
+  heads + CE / L1 / MSE -> trunk backward -> [two-arena peer exchange] -> Adam on the trunk and the branch arena, one CUDA
+  graph per input slot.
 * BranchedActStep -- its serving counterpart: stage [+ centre crop] -> conv1..4 -> the commanded branches -> greedy action,
   with the one-launch tail at small batch, one CUDA graph per input slot.
 * RolloutActStep -- serving N independent agents per tick: one new frame per agent staged into its on-device history,
@@ -306,12 +307,22 @@ class BranchedTrainStep(_BranchedInput, _GatherInput):
     of src_hw or 256x256, commands, and labels for 'ce' or targets for 'l1' / 'mse'); index (B,) int64 on the device;
     table (B, 8) f32 rows on the device when built with src_hw (row b for all four frames of sample b), else None. One
     bc_stage_gather launch stages the windows, commands and targets; one CUDA graph per (store, index buffer, table
-    buffer), which reads their contents on every replay."""
+    buffer), which reads their contents on every replay.
 
-    def __init__(self, net, optimizer, batch: int, *, src_hw=None, graph: bool = True, group=None):
-        if dist.is_initialized() and dist.get_world_size(group) > 1:
-            raise RuntimeError("BranchedTrainStep trains on one GPU: data-parallel training of the branched policy is not "
-                               "supported (the peer exchange drives a single parameter arena)")
+    Data parallel: when `group` (default: the whole torch.distributed world) has more than one rank, or with
+    exchange='peer' on any initialised group, each rank trains on its own shard at the same local batch, and the trunk
+    and branch gradients are written straight into peer-visible memory; one bc_adam_step_exchange_arenas launch inside the
+    graph sums them over the ranks in rank order and applies Adam to both arenas (parallel.BranchedPeerExchange), so the
+    replicas stay bitwise identical. 'peer' is the only exchange the branched policy has."""
+
+    def __init__(self, net, optimizer, batch: int, *, src_hw=None, graph: bool = True, group=None,
+                 exchange: Optional[str] = None):
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        if exchange not in (None, "peer"):
+            raise ValueError("the branched policy trains data-parallel with ddp_exchange 'peer' only (the two-arena exchange "
+                             "fused into the Adam kernel over NVLink peer memory)")
+        if exchange == "peer" and not dist.is_initialized():
+            raise RuntimeError("exchange='peer' needs an initialised torch.distributed process group")
         children = getattr(optimizer, "children_", None)
         if (children is None or len(children) != 2 or children[0]._arena_of is not net
                 or children[1]._arena_of is not net._bowner):
@@ -325,6 +336,11 @@ class BranchedTrainStep(_BranchedInput, _GatherInput):
         self.hb = dict(out=torch.empty((B, net.n_actions), **f32), dout=torch.empty((B, net.n_actions), **f32),
                        loss=torch.zeros((), **f32), grads=torch.zeros_like(net._barena),
                        partials=torch.zeros(n_part, **f32))     # partial pads are never written: zeroed once
+        self.dp = None
+        if world > 1 or exchange == "peer":         # data parallel: both arenas' gradients land in peer memory
+            from .parallel import BranchedPeerExchange
+            self.dp = BranchedPeerExchange(net, optimizer, group)
+            self.hb.update(self.dp.head_grads())
         optimizer.prepare()
         self._seen, self._graphs = set(), {}
 
@@ -348,8 +364,11 @@ class BranchedTrainStep(_BranchedInput, _GatherInput):
         self.eng.enqueue_trunk_forward(self.bufs)
         self.net._head(self.bufs, self.hb, command, target, 3)      # outputs, loss, dout, branch gradients, ghead
         self.eng.enqueue_trunk_backward(self.bufs)
-        self.trunk_opt.step_flat(self.eng.grads)
-        self.branch_opt.step_flat(self.hb["grads"])
+        if self.dp is not None:
+            self.dp.exchange()
+        else:
+            self.trunk_opt.step_flat(self.eng.grads)
+            self.branch_opt.step_flat(self.hb["grads"])
 
     # ------------------------------------------------------------------ step
     def step(self, frames_u8: torch.Tensor, table: Optional[torch.Tensor], command: torch.Tensor,
@@ -375,6 +394,8 @@ class BranchedTrainStep(_BranchedInput, _GatherInput):
             self._seen.add(key)
             self.opt.prepare()
             enqueue()
+        if self.dp is not None:
+            self.dp.peer.host_epoch += 1
         return self.hb["loss"]
 
     def step_gather(self, store, index: torch.Tensor, table: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -416,8 +437,11 @@ class BranchedTrainStep(_BranchedInput, _GatherInput):
         return self.hb["out"]
 
     def check(self) -> None:
-        """Raise if a device-side bounded wait expired, a label (CE) or a command was out of range (synchronises)."""
+        """Raise if a device-side bounded wait expired, a label (CE) or a command was out of range, or a peer rank never
+        arrived at the exchange (synchronises)."""
         self.eng.check_device_errors()
+        if self.dp is not None:
+            self.dp.peer.check()
 
 
 class BranchedActStep(_BranchedInput):
@@ -636,7 +660,13 @@ class Trainer:
         opt, self._opt, self._schedulers = optimizers[0], optimizers[0], schedulers
         net = getattr(model, "net", None)
         world = dist.get_world_size() if dist.is_initialized() else 1
-        if world > 1:
+        if world > 1 and getattr(opt, "children_", None) is not None:       # the branched policy's MultiArenaAdam
+            if self.ddp_exchange != "peer":
+                raise RuntimeError("the branched policy trains data-parallel with ddp_exchange 'peer' only (the two-arena "
+                                   f"exchange fused into the Adam kernel), got {self.ddp_exchange!r}")
+            from .parallel import BranchedPeerExchange
+            BranchedPeerExchange(net, opt)
+        elif world > 1:
             if not isinstance(opt, FusedAdam):
                 raise RuntimeError("data-parallel training needs the arena-backed FusedAdam (ConvNet1 parameters)")
             if self.ddp_exchange == "peer":

@@ -243,6 +243,16 @@ typedef struct {
 } bc_peer;
 int bc_adam_step_exchange(float* params, float* exp_avg, float* exp_avg_sq, double* state9, int64_t n, const bc_peer* peer,
                           int64_t lo, int64_t hi, int bucket, int publish, void* w_packed, int obs_size, int n_actions, void* stream);
+/* The same exchange for two parameter arenas in ONE launch (the branched policy: trunk arena + branch arena): each rank's
+ * gradient buffer holds two halves of n floats (stride n), each half = [arena 0: split floats | arena 1: n - split floats].
+ * One flag round trip (bucket 1 slots), the rank-order sum of the whole half, Adam on arena 0 with (params, exp_avg,
+ * exp_avg_sq, state9) and on arena 1 with the _b set, each with its own state (grad_scale, lr, step); w_packed refreshes the
+ * operand images of arena 0 only (split must then be the arena of (obs_size, n_actions)). The last CTA publishes both ticks
+ * and the epoch. Do not call bc_adam_tick for either state. */
+int bc_adam_step_exchange_arenas(float* params, float* exp_avg, float* exp_avg_sq, double* state9,
+                                 float* params_b, float* exp_avg_b, float* exp_avg_sq_b, double* state9_b,
+                                 int64_t n, int64_t split, const bc_peer* peer, void* w_packed, int obs_size, int n_actions,
+                                 void* stream);
 
 /* ---- K12: Imitation.forward + argmax (imitation.py:34-36, src/data/stat.py:41). Every greedy action of this library
  * (bc_argmax, bc_forward_act on both paths) follows torch.argmax: the index of the first NaN of the row if it has one (NaN
@@ -292,6 +302,10 @@ typedef struct {
     float* partials;          /* bc_head_branched_partials_floats() floats */
     int32_t* err_flag;        /* 3 = label out of range, 4 = command out of range */
     float loss_scale;
+    const uint32_t* grads_epoch; /* data-parallel peer exchange only (else NULL): as bc_ctx.grads_epoch -- the backward (bit1)
+                                    writes the branch gradients to grads + ((*grads_epoch + 1) & 1) * grads_stride, the half
+                                    bc_adam_step_exchange_arenas reads next                                                 */
+    int64_t grads_stride;     /* floats between the two halves                                                           */
 } bc_branched;
 int bc_head_branched(const bc_branched* h, int mode, void* stream);
 size_t bc_head_branched_partials_floats(int n_branches, int n_out);

@@ -146,6 +146,8 @@ class ConvNet1Branched(ConvNet1):
         h.out, h.dout, h.loss = hb["out"].data_ptr(), hb["dout"].data_ptr(), hb["loss"].data_ptr()
         h.gfeat = bufs.ghead.data_ptr() if bufs.ghead is not None else None
         h.partials, h.err_flag = hb["partials"].data_ptr(), eng.err_flag.data_ptr()
+        if hb.get("grads_epoch") is not None:     # data parallel: the branch gradients go to the peer half of this step
+            h.grads_epoch, h.grads_stride = hb["grads_epoch"].data_ptr(), hb["grads_stride"]
         n = max(bufs.batch, 1) * (1 if self.branch_loss == "ce" else self.n_actions)
         h.loss_scale = 1.0 / n
         with torch.cuda.device(eng.device):
@@ -257,6 +259,7 @@ class MultiArenaAdam(torch.optim.Optimizer):
         super().__init__(params, dict(lr=lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False))
         self.children_ = [FusedAdam(list(ps), lr=lr) for ps in param_lists]
         self._linked = [None] * len(self.children_)
+        self.exchange = None          # parallel.BranchedPeerExchange when the module path trains data-parallel
 
     def _link_state(self) -> None:
         """self.state[p] = the child's torch.optim.Adam-compatible views (FusedAdam._bind), refreshed when a child rebinds."""
@@ -272,9 +275,17 @@ class MultiArenaAdam(torch.optim.Optimizer):
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
-        for c in self.children_:
-            c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
-            c.step()
+        if self.exchange is not None:          # data parallel: both arenas' gradients -> one exchange launch
+            grads = []
+            for c in self.children_:
+                c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
+                arena, _m, _v, _st, flat_g = c._bind()
+                grads.append(c._flat_grads(arena, flat_g))
+            self.exchange.step_from(*grads)
+        else:
+            for c in self.children_:
+                c.param_groups[0]["lr"] = self.param_groups[0]["lr"]
+                c.step()
         self._link_state()
         return loss
 
